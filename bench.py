@@ -8,7 +8,7 @@ shard that is already resident in HBM: K1 (FFT, samples -> N complex bins), K3 (
 record) and - for G > 1 - the records reaching rank 0 (K3 stores them straight into rank 0's table over NVLink; the
 NCCL gather is the alternative, --gather nccl).  No collective touches the data path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 Extra keys of the line: roofline (dominant kernel K1, timed live with CUDA events), pipeline (whole step vs B_alg),
@@ -63,7 +63,13 @@ def parse_args():
     ap.add_argument("--no-variants", action="store_true")
     ap.add_argument("--no-configs", action="store_true")
     ap.add_argument("--no-numa", action="store_true", help="do not bind the process to the GPU's NUMA node")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy: the peak records of "
+                         "a fixed, seeded sample of windows and the spectra of a smaller such sample (at most 64 MB)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 # ---------------------------------------------------------------------------------------------------------------
@@ -479,6 +485,8 @@ def run_ours(args):
     launches0 = an.launch_count()
     step_ms, k1_ms, clocks, table = fleet.timed(args.steps, warm)
     launches = (an.launch_count() - launches0) * args.steps // (args.steps + warm)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, table[:total], fleet.d_spec[:b])
 
     # ---- the table of one more step, and its NCCL twin (hard check on every multi-GPU run) -------------------------
     nccl_equal = None
@@ -734,6 +742,44 @@ def run_ours(args):
     if failed:
         sys.stderr.write("bench.py: the peer-memory record table differs from the NCCL gather\n")
         sys.exit(3)
+
+
+DUMP_SEED = 20261020
+DUMP_RECORD_WINDOWS = 131072        # 184 bytes each as float64: 24 MB
+DUMP_SPECTRUM_BYTES = 32 << 20
+
+
+def dump_outputs(out_dir, table, spectra):
+    """Write the headline step's outputs as <out_dir>/<name>.npy, so that two builds can be compared output for output.
+
+    table: uint8 [windows, 128] records of the whole fleet (window order); spectra: [rows, N, 2] of rank 0's shard,
+    whose first row is window 0.  The samples depend only on the shapes, so the same arguments pick the same windows.
+      record_window, record_count, record_status  float64 [R]      window ids, peaks found, status bits
+      peak_idx, peak_width_bins, peak_mag,        float64 [R, 5]   the record's peak slots (idx -1: empty)
+      peak_prominence
+      spectrum_window                             float64 [S]      window ids of the spectrum sample
+      spectrum                                    [S, N, 2]        K1's complex bins in the compute dtype
+    """
+    import numpy as np
+    import torch
+    from apda_fft_b200.records import record_dtype
+
+    os.makedirs(out_dir, exist_ok=True)
+    rng = np.random.default_rng(DUMP_SEED)
+    windows = table.shape[0]
+    pick = np.sort(rng.choice(windows, min(windows, DUMP_RECORD_WINDOWS), replace=False))
+    recs = table[torch.from_numpy(pick).to(table.device)].cpu().numpy().view(record_dtype(5)).reshape(-1)
+    out = {"record_window": pick, "record_count": recs["count"], "record_status": recs["status"],
+           "peak_idx": recs["pk"]["idx"], "peak_width_bins": recs["pk"]["width_bins"], "peak_mag": recs["pk"]["mag"],
+           "peak_prominence": recs["pk"]["prominence"]}
+    out = {name: np.ascontiguousarray(v, dtype=np.float64) for name, v in out.items()}
+    rows = spectra.shape[0]
+    row_bytes = spectra[0].numel() * spectra.element_size() if rows else 1
+    pick = np.sort(rng.choice(rows, min(rows, DUMP_SPECTRUM_BYTES // row_bytes), replace=False))
+    out["spectrum_window"] = pick.astype(np.float64)
+    out["spectrum"] = spectra[torch.from_numpy(pick).to(spectra.device)].cpu().numpy()
+    for name, v in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), v)
 
 
 def run_configs(an, dev, stream, sampler, peak):

@@ -236,14 +236,28 @@ def isclose_rel(a, b, tol):
     return approx_rel(float(a), float(b)) <= tol or (math.isnan(a) and math.isnan(b))
 
 
-def write_sensor_log(path, samples, fs: float, axis: str, per_line: int = 60, missing_marker_at: int | None = None) -> None:
-    """A sensor .log as the gateway writes it (GT_FFT_v5.py:380-395 header lines, protocol_decoder.py:174 "%8.6f"
-    samples, ';'-separated): what utils/load_data.py:29-82 parses."""
-    rows = [f"2_11_22_18_20_32;2 g;{fs} Hz;{axis} axis;", "Synced;", "25.010;-0.0222;0.0110;0.9981;85.0;",
-            "0.268262;0.0;1.0;"]
-    vals = ["%8.6f" % v for v in samples]
-    rows += [";".join(vals[i:i + per_line]) + ";" for i in range(0, len(vals), per_line)]
-    if missing_marker_at is not None:
-        rows.insert(missing_marker_at, "* MISSING PACKETS 3-4 *")
-    with open(path, "w") as fh:
-        fh.write("\n".join(rows) + "\n")
+def fuzz_inputs(seed, count):
+    """Deterministic adversarial inputs: ties, plateaus, odd lengths, DC offsets, spiky magnitude spectra."""
+    rng = np.random.default_rng(seed)
+    for i in range(count):
+        n = int(rng.integers(1, 70)) if i % 3 else int(rng.choice([2, 3, 4, 7, 8, 16, 31, 32, 64, 100, 128, 200, 256]))
+        kind = i % 4
+        if kind == 0:
+            x = np.round(rng.standard_normal(n), 1)                       # many ties
+        elif kind == 1:
+            x = np.round(np.sin(np.arange(n) * rng.uniform(0.1, 2.5)) + 0.05 * rng.standard_normal(n) + rng.uniform(-3, 3), 6)
+        elif kind == 2:
+            x = rng.integers(-3, 4, n).astype(np.float64)                 # plateaus, repeated medians
+        else:
+            x = np.round(np.exp(rng.standard_normal(n)), 3)               # skewed
+        yield x.tolist()
+
+
+def fuzz_spectra(seed, count):
+    rng = np.random.default_rng(seed)
+    for i in range(count):
+        n = int(rng.choice([8, 16, 32, 64, 128, 256]))
+        mags = np.round(np.exp(1.4 * rng.standard_normal(n)), int(rng.integers(0, 4)))   # rounded: equal neighbours occur
+        mags[0] = 0.0
+        phase = np.exp(1j * rng.uniform(0, 2 * np.pi, n)) if i % 2 else np.ones(n)
+        yield (mags * phase).tolist(), float(rng.choice([31.25, 62.5, 125.0, 250.0, 500.0])), int(rng.integers(1, 8))

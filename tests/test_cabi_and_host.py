@@ -145,19 +145,13 @@ def test_load_sensor(tmp_path):
     got = load_sensor(str(path))
     assert got["metadata"] == {"timestamp": "2_11_22_18_20_32", "sensitivity": "2g", "fs": 31.25, "axis": "Z",
                                "sync_type": "Synced2", "is_synced": 1.0}
+    assert list(got["metadata"]) == ["timestamp", "sensitivity", "fs", "axis", "sync_type", "is_synced"]
     assert got["summary"] == {"temperature": 25.01, "rms_x": -0.0222, "rms_y": 0.011, "rms_z": 0.9981, "humidity": 85.0,
                               "first_x": 0.268262, "first_y": -0.5, "first_z": 1.0}
     assert got["samples"] == [0.1, 0.2, -0.3, 0.4, 0.5, -0.0, 1000.0]
     short = tmp_path / "b.log"
     short.write_text("a;b;1 Hz;X axis;\nNo;\n")
     assert load_sensor(str(short)) is None
-    if os.path.isdir("/root/reference"):        # live cross-check in the build container
-        import importlib.util
-        spec = importlib.util.spec_from_file_location("_ref_load_data", "/root/reference/utils/load_data.py")
-        mod = importlib.util.module_from_spec(spec)
-        spec.loader.exec_module(mod)
-        assert mod.load_sensor(str(path)) == got and list(mod.load_sensor(str(path))["metadata"]) == list(got["metadata"])
-        assert mod.load_sensor(str(short)) is None
 
 
 def test_pure_host_helpers():
@@ -213,7 +207,6 @@ def test_c_host_example_compiles_and_links(lib, tmp_path):
 def test_result_packing_arrow_jsonl_and_upload_metrics(golden, tmp_path):
     """SURVEY 8f rank 4: columnar / JSONL packing of a record batch and the uploader's `metriche` block."""
     import json
-    import subprocess
     from apda_fft_b200.records import (fleet_arrow, gateway_entry, record_dtype, upload_metrics, write_fleet_jsonl,
                                        prominence_dicts)
     recs = np.zeros(3, dtype=record_dtype(5))
@@ -240,15 +233,9 @@ def test_result_packing_arrow_jsonl_and_upload_metrics(golden, tmp_path):
     entry = gateway_entry(golden["cases"]["katA"]["prominence"]["ok"])
     got = upload_metrics(summary, "Z", entry)
     assert got["rms_asse"] == 0.9981 and got["fft_freqs"][:3] == [3.0518, 7.6904, 15.1367] and got["fft_freqs"][3] == 0.0
-    if os.path.isdir("/root/reference"):   # the live uploader's payload for the same file and fft_dict entry
-        log = os.path.join(str(tmp_path), "0013a20041e7f6b7_01_02_2024_03_04_05_Zaxis.log")
-        with open(log, "w") as fh:
-            fh.write(LOG_TEXT.replace("31.25 Hz;Z axis", "125.0 Hz;Z axis"))
-        code = ("import json,sys; sys.path.insert(0, '/root/reference'); from utils.fastapi_manager import FastAPIHandler; "
-                f"p = FastAPIHandler('x')._prepare_payload('mac', {os.path.basename(log)!r}, {str(tmp_path)!r}, "
-                f"{{'Z': {entry!r}}}); print(json.dumps(p['metriche']))")
-        ref = json.loads(subprocess.check_output([sys.executable, "-c", code], text=True))
-        assert ref == json.loads(json.dumps(got))
+    assert got == {"temp": 25.01, "humidity": 85.0, "phi": 153.64179189369935, "theta": 1.4219587307998718,
+                   "rms_asse": 0.9981, "fft_freqs": [3.0518, 7.6904, 15.1367, 0.0],
+                   "fft_mags": [195.833, 149.3667, 65.4201, 0.0]}
 
 
 def test_dropins_never_hand_out_a_record_with_nonzero_status():

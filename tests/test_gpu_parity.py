@@ -688,7 +688,7 @@ def _outcome(fn, *args, **kw):
 
 
 def test_fuzz_small_windows_and_spectra_vs_oracle(an):
-    """The adversarial inputs that pin the oracle to the live reference (tests/test_oracle.py: 400 windows of length
+    """The adversarial inputs that pinned the oracle to the live reference (tests/cases.py: 400 windows of length
     1..256 with ties / plateaus / offsets, 300 hand-shaped spectra with k = 1..7) through the drop-in modules, i.e.
     the reference's own call signatures on the CUDA path: spectra equal element by element (fp64 bit-exact), peak
     lists equal objects, same exception types for degenerate sizes."""
@@ -697,14 +697,13 @@ def test_fuzz_small_windows_and_spectra_vs_oracle(an):
     from metrics.fft_iterativa import start_fft
     from utils.get_peak_prominence import get_top_peaks_prominence
     from utils.get_peak_resolution import get_top_peaks_resolution
-    from test_oracle import _fuzz_inputs, _fuzz_spectra
-    for x in _fuzz_inputs(20260101, 400):
+    for x in cases.fuzz_inputs(20260101, 400):
         want = ref_port.start_fft(list(x), 125.0)
         got = start_fft(list(x), 125.0)
         assert len(got) == len(want) and all(complex(a) == complex(b) for a, b in zip(got, want)), x
         assert _outcome(get_top_peaks_prominence, got, 125.0) == _outcome(ref_port.top_peaks_prominence, list(want), 125.0), x
         assert _outcome(get_top_peaks_resolution, got, 125.0) == _outcome(ref_port.top_peaks_resolution, list(want), 125.0), x
-    for spec, fs, k in _fuzz_spectra(7, 300):
+    for spec, fs, k in cases.fuzz_spectra(7, 300):
         assert _outcome(get_top_peaks_prominence, list(spec), fs, k) == _outcome(ref_port.top_peaks_prominence, list(spec), fs, k)
         assert _outcome(get_top_peaks_resolution, list(spec), fs, k) == _outcome(ref_port.top_peaks_resolution, list(spec), fs, k)
 

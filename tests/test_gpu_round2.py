@@ -1,6 +1,5 @@
 """T2, second round: the parity holes the round-1 review listed (needs a B200: -m gpu).
 
-  * the UNMODIFIED reference call site Gateway.work_flow_fft on the drop-in modules (SURVEY 8 row a12),
   * multi-chunk host pipelines with pinned buffers where both pipeline streams use the device-side window lists
     (repair list of the fast pickers, ragged list of the ingest paths) at the same time,
   * record status bits on every ragged path, any k through the drop-ins, the fp32 tie flag,
@@ -10,14 +9,13 @@
 import ctypes
 import json
 import os
-import subprocess
 import sys
 
 import numpy as np
 import pytest
 
 import cases
-from oracle import c_oracle, ref_copy, ref_port
+from oracle import c_oracle, ref_port
 
 pytestmark = pytest.mark.gpu
 
@@ -34,52 +32,6 @@ def an():
 def _dicts(rec, fs, n, flexible):
     from apda_fft_b200.records import prominence_dicts, resolution_dicts
     return prominence_dicts(rec, fs, n) if flexible else resolution_dicts(rec, fs, n)
-
-
-# ---------------------------------------------------------------------------------------------------------------
-# a12: the reference's own caller, unmodified, on the drop-ins
-# ---------------------------------------------------------------------------------------------------------------
-TIMING_KEYS = ("process_time", "wall_time", "percentage_cpu", "memrss")
-
-
-def _replay(mode, flexible, mac, paths):
-    out = subprocess.run([sys.executable, os.path.join(ROOT, "tests", "gateway_replay.py"), mode, str(int(flexible)), mac, *paths],
-                         capture_output=True, text=True, timeout=600)
-    assert out.returncode == 0, out.stderr[-2000:]
-    assert "[ERROR]" not in out.stdout, out.stdout[-2000:]          # work_flow_fft's broad except only prints
-    return json.loads(out.stdout.strip().splitlines()[-1])
-
-
-@pytest.mark.parametrize("flexible", [True, False])
-def test_gateway_work_flow_fft_unmodified_call_site(flexible, tmp_path, golden):
-    """GT_FFT_v5.py:620-680 from the build-time copy of the reference (oracle/_ref), digidevice stubbed, run once on
-    the reference's own hot-path modules and once with apda-fft_b200/ ahead on sys.path (INTEGRATION.md): the fft_dict
-    entries must be the same Python objects (every key but the caller's own timing fields), for both values of
-    is_flexibile_structure, on KAT-A/B/C logs (one file per axis, one of them with a MISSING PACKETS marker)."""
-    if not ref_copy.available(call_site=True):
-        pytest.skip("oracle/_ref is not populated (built only where /root/reference exists)")
-    mac = "0013a20041e7f6b7"
-    paths = []
-    for axis, cid, marker in (("X", "katA", 9), ("Y", "katB", None), ("Z", "katC", 30)):
-        x, fs = cases.build_samples(golden["cases"][cid]["spec"])
-        path = tmp_path / f"{mac}_{axis}axis.log"
-        cases.write_sensor_log(path, x, fs, axis, missing_marker_at=marker)
-        paths.append(str(path))
-    ref = _replay("ref", flexible, mac, paths)
-    new = _replay("dropin", flexible, mac, paths)
-    assert ref["gateway"] == new["gateway"] == "oracle/_ref/GT_FFT_v5.py"
-    assert ref["bound"] == "oracle/_ref/metrics/fft_iterativa.py"
-    assert new["bound"] == "apda-fft_b200/metrics/fft_iterativa.py"
-    assert set(new["fft_dict"][mac]) == {"X", "Y", "Z"}
-    for axis in "XYZ":
-        a, b = ref["fft_dict"][mac][axis], new["fft_dict"][mac][axis]
-        assert set(a) == set(b)
-        for key in a:
-            if key not in TIMING_KEYS:
-                assert a[key] == b[key], (axis, key, a[key], b[key])
-        assert b["peak_freq"] != -1 and "peak_freq_3" in b
-    want = golden["cases"]["katA"]["prominence" if flexible else "resolution"]["ok"]
-    assert new["fft_dict"][mac]["X"]["peak_freq_1"] == want[0]["freq"]
 
 
 # ---------------------------------------------------------------------------------------------------------------
