@@ -1,4 +1,4 @@
-// K2: multi-pass FFT for transforms that exceed shared memory (N > 2^13 fp64 / 2^14 fp32, up to 2^30).
+// K2: multi-pass FFT for transforms longer than 2^13 in both precisions (N = 2^14 ... 2^30, any batch).
 //
 // The reference's radix-2 DIT dataflow graph (metrics/fft_iterativa.py:38-70) is cut into P passes of q_p stages
 // (sum q_p = log2 N, q_p <= 10 fp64 / 11 fp32).  Every pass moves the data through HBM exactly once:
@@ -1119,51 +1119,12 @@ static int launch_head(apda_ctx *ctx, cudaStream_t st, dim3 grid, size_t smem, c
     return APDA_OK;
 }
 
-}  // namespace
-
+// head pass and tail passes of `batch` <= 65535 windows (gridDim.y); d_med: the windows' centring constants or NULL
 template <typename T>
-int launch_fft_large(apda_ctx *ctx, cudaStream_t st, const T *d_samples, int64_t n_samples, int64_t ld, int64_t batch,
-                     int64_t N, int flags, T *d_spec, bool complex_input) {
+static int large_passes(apda_ctx *ctx, cudaStream_t st, const T *d_samples, int64_t n_samples, int64_t ld, int64_t batch, int n,
+                        const PassPlan &plan, int max_tile, const K2Tune &tune, const typename vec2<T>::type *twp, T *d_spec,
+                        const T *d_med, bool complex_input) {
     using V2 = typename vec2<T>::type;
-    const int n = ilog2_i64(N);
-    if (n > 30 || batch > 65535) {
-        apda_set_error("fft_large: N=2^%d batch=%lld outside the supported range", n, (long long)batch);
-        return APDA_ERR_UNSUPPORTED;
-    }
-    TwiddleTables tw;
-    APDA_TRY(apda_get_twiddles(ctx, N, &tw));
-    const V2 *twp = sizeof(T) == 8 ? reinterpret_cast<const V2 *>(tw.d64) : reinterpret_cast<const V2 *>(tw.d32);
-    const K2Tune tune = k2_tune<T>();
-    const int max_tile = tune.max_tile;  // complex elements per tile: 64 KB tiles let 3 CTAs per SM overlap load, compute and store
-    const PassPlan plan = make_plan(n, tune.qmax);
-
-    // centring constant per window
-    T *d_med = nullptr;
-    if (!complex_input && flags != APDA_CENTER_NONE) {
-        // per-stream scratch: the two host-pipeline streams may run long transforms concurrently
-        const size_t med_bytes = ((size_t)batch * sizeof(T) + 255) & ~(size_t)255;
-        const int64_t wins = ctx->generic_only ? 1 : median_windows<T>(n_samples, batch);
-        const size_t state_bytes = (std::max(sizeof(BracketState<T>) * (size_t)wins, sizeof(SelectState)) + 255) & ~(size_t)255;
-        // states, medians, bucket copies (worst case: all samples of every window of a launch set)
-        const size_t need = state_bytes + med_bytes + (size_t)wins * (size_t)n_samples * sizeof(T);
-        auto &slot = ctx->stream_scratch[st];
-        if (need > slot.second) {
-            APDA_CUDA(cudaStreamSynchronize(st));
-            APDA_TRY(apda_reserve(&slot.first, &slot.second, need));
-        }
-        SelectState *state = reinterpret_cast<SelectState *>(slot.first);
-        d_med = reinterpret_cast<T *>(reinterpret_cast<char *>(slot.first) + state_bytes);
-        T *d_bucket = reinterpret_cast<T *>(reinterpret_cast<char *>(slot.first) + state_bytes + med_bytes);
-        if (ctx->generic_only) {
-            for (int64_t w = 0; w < batch; ++w)
-                APDA_TRY(large_median_passes<T>(ctx, st, d_samples + w * ld, n_samples, state, d_med + w));
-        } else {
-            for (int64_t w0 = 0; w0 < batch; w0 += wins)
-                APDA_TRY(large_median<T>(ctx, st, d_samples + w0 * ld, n_samples, ld, std::min<int64_t>(wins, batch - w0), slot.first,
-                                         d_med + w0, d_bucket));
-        }
-    }
-
     {  // head pass
         const int q = plan.q[0];
         const int64_t cols = (int64_t)1 << (n - q);
@@ -1217,6 +1178,64 @@ int launch_fft_large(apda_ctx *ctx, cudaStream_t st, const T *d_samples, int64_t
         ctx->launches++;
         APDA_CUDA(cudaGetLastError());
         s0 += q;
+    }
+    return APDA_OK;
+}
+
+}  // namespace
+
+template <typename T>
+int launch_fft_large(apda_ctx *ctx, cudaStream_t st, const T *d_samples, int64_t n_samples, int64_t ld, int64_t batch,
+                     int64_t N, int flags, T *d_spec, bool complex_input) {
+    using V2 = typename vec2<T>::type;
+    const int n = ilog2_i64(N);
+    if (n > 30) {
+        apda_set_error("fft_large: N=2^%d outside the supported range", n);
+        return APDA_ERR_UNSUPPORTED;
+    }
+    TwiddleTables tw;
+    APDA_TRY(apda_get_twiddles(ctx, N, &tw));
+    const V2 *twp = sizeof(T) == 8 ? reinterpret_cast<const V2 *>(tw.d64) : reinterpret_cast<const V2 *>(tw.d32);
+    const K2Tune tune = k2_tune<T>();
+    const int max_tile = tune.max_tile;  // complex elements per tile: 64 KB tiles let 3 CTAs per SM overlap load, compute and store
+    const PassPlan plan = make_plan(n, tune.qmax);
+
+    // centring constant per window
+    T *d_med = nullptr;
+    if (!complex_input && flags != APDA_CENTER_NONE) {
+        // per-stream scratch: the two host-pipeline streams may run long transforms concurrently
+        const size_t med_bytes = ((size_t)batch * sizeof(T) + 255) & ~(size_t)255;
+        const int64_t wins = ctx->generic_only ? 1 : median_windows<T>(n_samples, batch);
+        const size_t state_bytes = (std::max(sizeof(BracketState<T>) * (size_t)wins, sizeof(SelectState)) + 255) & ~(size_t)255;
+        // states, medians, bucket copies (worst case: all samples of every window of a launch set)
+        const size_t need = state_bytes + med_bytes + (size_t)wins * (size_t)n_samples * sizeof(T);
+        auto &slot = ctx->stream_scratch[st];
+        if (need > slot.second) {
+            APDA_CUDA(cudaStreamSynchronize(st));
+            APDA_TRY(apda_reserve(&slot.first, &slot.second, need));
+        }
+        SelectState *state = reinterpret_cast<SelectState *>(slot.first);
+        d_med = reinterpret_cast<T *>(reinterpret_cast<char *>(slot.first) + state_bytes);
+        T *d_bucket = reinterpret_cast<T *>(reinterpret_cast<char *>(slot.first) + state_bytes + med_bytes);
+        if (ctx->generic_only) {
+            for (int64_t w = 0; w < batch; ++w)
+                APDA_TRY(large_median_passes<T>(ctx, st, d_samples + w * ld, n_samples, state, d_med + w));
+        } else {
+            for (int64_t w0 = 0; w0 < batch; w0 += wins)
+                APDA_TRY(large_median<T>(ctx, st, d_samples + w0 * ld, n_samples, ld, std::min<int64_t>(wins, batch - w0), slot.first,
+                                         d_med + w0, d_bucket));
+        }
+    }
+
+    // head and tail passes put the windows on gridDim.y (at most 65535): longer batches run in launch sets of that many
+    // windows, each with its own samples, spectra, centring constants and tensor maps
+    constexpr int64_t kMaxSet = 65535;
+    for (int64_t w0 = 0; w0 < batch; w0 += kMaxSet) {
+        const int64_t wb = std::min<int64_t>(kMaxSet, batch - w0);
+        const T *x = d_samples + w0 * (complex_input ? 2 * N : ld);
+        T *y = d_spec + w0 * 2 * N;
+        const T *med = d_med ? d_med + w0 : nullptr;
+        APDA_TRY(large_passes<T>(ctx, st, x, n_samples, ld, wb, n, plan, max_tile, tune, twp, y, med, complex_input));
     }
     return APDA_OK;
 }

@@ -90,7 +90,8 @@ int64_t apda_launch_count(apda_ctx *ctx);
  * replaces metrics/fft_iterativa.py:74-87 start_fft(samples, fs): median centre (:5-11), zero pad (:13-22),
  * bit reversal (:24-36), radix-2 DIT butterflies with the recurrence twiddles (:38-70), bin 0 := 0 (:85).
  * f64 is bit-faithful to the reference (no FMA, host-built recurrence twiddle table).  f32 is the fast path.
- * N <= 2^13 (f64) / 2^14 (f32) runs one shared-memory kernel per window batch; larger N runs the multi-pass kernels. */
+ * N <= 2^13 runs one shared-memory kernel per window batch in both precisions; N = 2^14 ... 2^30 runs the multi-pass
+ * kernels (K2), for any batch.  fp32 N = 2^14 fits the shared-memory kernel too, but only ragged batches use it there. */
 int apda_fft_f64_dev(apda_ctx *ctx, const double *d_samples, int64_t n_samples, int64_t ld, int64_t batch,
                      int64_t N, int flags, double *d_spec);
 int apda_fft_f32_dev(apda_ctx *ctx, const float *d_samples, int64_t n_samples, int64_t ld, int64_t batch,
