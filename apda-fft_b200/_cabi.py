@@ -67,6 +67,8 @@ SIGNATURES = {
     "apda_analyze_text_f32_host": (_int, [_p, _p, _p, _i64, _i64, _i64, _int, _int, _dbl, _p, _int, _int, _p, _p, _p]),
     "apda_analyze_fused_f32_dev": (_int, [_p, _p, _i64, _i64, _i64, _i64, _int, _int, _dbl, _p, _int, _int, _p]),
     "apda_analyze_fused_f32_host": (_int, [_p, _p, _i64, _i64, _i64, _i64, _int, _int, _dbl, _p, _int, _int, _p]),
+    "apda_resolve_fp32_ties_dev": (_int, [_p, _p, _p, _i64, _i64, _i64, _i64, _int, _int, _dbl, _p, _int, _int, _p]),
+    "apda_resolve_fp32_ties_host": (_int, [_p, _p, _p, _i64, _i64, _i64, _i64, _int, _int, _dbl, _p, _int, _int, _p]),
     "apda_prominence_f64_host": (_int, [_p, _p, _i64, _i64, _c.POINTER(_dbl)]),
     "apda_half_power_bins_f64_host": (_int, [_p, _p, _i64, _dbl, _i64, _c.POINTER(_i64)]),
     "apda_half_height_bins_f64_host": (_int, [_p, _p, _i64, _i64, _c.POINTER(_i64)]),

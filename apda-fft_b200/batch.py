@@ -73,7 +73,7 @@ class Analyzer:
                 n_fft: int | None = None, center: int = _cabi.CENTER_MEDIAN, rec_cap: int | None = None,
                 resolve_ties: bool = True) -> np.ndarray:
         """[B, n_samples] real (float32 or float64) -> records[B]; spectra never leave the device.  float32 windows
-        whose record carries APDA_STATUS_FP32_TIE are re-run in float64 (``resolve_ties``)."""
+        whose record status is APDA_STATUS_FP32_TIE get the float64 path's record (``resolve_ties``)."""
         x = np.ascontiguousarray(np.atleast_2d(samples))
         sfx = _suffix(x.dtype)
         b, ns = x.shape
@@ -85,22 +85,22 @@ class Analyzer:
         self.ctx.call(f"apda_analyze_{sfx}_host", _p(x.ctypes.data), ns, ns, b, n, center, int(bool(flexible)),
                       fs_scalar, _p(fs_arr.ctypes.data if fs_arr is not None else 0), k, cap, _p(recs.ctypes.data))
         if sfx == "f32" and resolve_ties:
-            self._resolve_fp32_ties(x, recs, fs, flexible, k, n, cap)
+            self._resolve_fp32_ties(x, recs, fs, flexible, k, n, cap, center)
         return recs
 
-    def _resolve_fp32_ties(self, x, recs, fs, flexible, k, n, cap) -> int:
+    def _resolve_fp32_ties(self, x, recs, fs, flexible, k, n, cap, center) -> None:
         """Windows flagged APDA_STATUS_FP32_TIE (two equal fp32 magnitudes at a peak top: no strict local maximum, so
-        the fp32 picker dropped a peak the fp64 reference reports) are re-run through the fp64 pipeline on the same
-        samples and their records replaced.  About one window in 10^6 of the fleet generator."""
-        tied = np.flatnonzero(recs["status"] & _cabi.STATUS_FP32_TIE)
-        if tied.size:
-            fs_sel = fs if np.isscalar(fs) else np.asarray(fs, dtype=np.float64)[tied]
-            recs[tied] = self.analyze(x[tied].astype(np.float64), fs_sel, flexible=flexible, k=k, n_fft=n, rec_cap=cap)
-        return int(tied.size)
+        the fp32 picker dropped a peak the fp64 reference reports) get the record the fp64 path computes from the same
+        samples with the same centring (apda_resolve_fp32_ties_host).  About one window in 10^6 of the fleet generator."""
+        b, ns = x.shape
+        fs_scalar, fs_arr = self._fs(fs, b)
+        self.ctx.call("apda_resolve_fp32_ties_host", _p(x.ctypes.data), _p(0), ns, ns, b, n, center, int(bool(flexible)),
+                      fs_scalar, _p(fs_arr.ctypes.data if fs_arr is not None else 0), k, cap, _p(recs.ctypes.data))
 
     def analyze_fused(self, samples: np.ndarray, fs, flexible: bool = True, k: int | None = None,
-                      center: int = _cabi.CENTER_MEDIAN) -> np.ndarray:
-        """[B, N] float32, N in {1024, 2048, 4096, 8192} -> records[B] through the fused window->record kernel."""
+                      center: int = _cabi.CENTER_MEDIAN, resolve_ties: bool = False) -> np.ndarray:
+        """[B, N] float32, N in {1024, 2048, 4096, 8192} -> records[B] through the fused window->record kernel
+        (``resolve_ties``: then the fp64 path's records for the windows flagged APDA_STATUS_FP32_TIE)."""
         x = np.ascontiguousarray(np.atleast_2d(samples), dtype=np.float32)
         b, ns = x.shape
         n = next_pow2(ns)
@@ -109,13 +109,18 @@ class Analyzer:
         fs_scalar, fs_arr = self._fs(fs, b)
         self.ctx.call("apda_analyze_fused_f32_host", _p(x.ctypes.data), ns, ns, b, n, center, int(bool(flexible)), fs_scalar,
                       _p(fs_arr.ctypes.data if fs_arr is not None else 0), k, 5, _p(recs.ctypes.data))
+        if resolve_ties:
+            self._resolve_fp32_ties(x, recs, fs, flexible, k, n, 5, center)
         return recs
 
     def analyze_fused_device(self, d_samples: int, batch: int, n_samples: int, n_fft: int, fs: float, d_rec: int,
                              flexible: bool = True, k: int = 4, center: int = _cabi.CENTER_MEDIAN, d_fs: int = 0,
-                             ld: int | None = None) -> None:
+                             ld: int | None = None, resolve_ties: bool = False) -> None:
         self.ctx.call("apda_analyze_fused_f32_dev", _p(d_samples), n_samples, ld or n_samples, batch, n_fft, center,
                       int(bool(flexible)), float(fs), _p(d_fs), k, 5, _p(d_rec))
+        if resolve_ties:
+            self.resolve_fp32_ties_device(d_samples, batch, n_samples, n_fft, fs, d_rec, flexible, k, 5, center, d_fs,
+                                          0, ld)
 
     # ---- wire-format ingest (16-bit samples, high byte first) ----------------------------------------------------------
     def decode_wire16(self, payload: np.ndarray, first_value) -> tuple[np.ndarray, np.ndarray]:
@@ -174,9 +179,22 @@ class Analyzer:
 
     def analyze_device(self, d_samples: int, batch: int, n_samples: int, n_fft: int, dtype: str, fs: float, d_rec: int,
                        flexible: bool = True, k: int = 4, rec_cap: int = 5, center: int = _cabi.CENTER_MEDIAN,
-                       d_spec_ws: int = 0, d_fs: int = 0, ld: int | None = None) -> None:
+                       d_spec_ws: int = 0, d_fs: int = 0, ld: int | None = None, resolve_ties: bool = False) -> None:
+        """``resolve_ties`` (float32 only): then the fp64 path's records for the windows flagged APDA_STATUS_FP32_TIE,
+        enqueued on the same stream (apda_resolve_fp32_ties_dev)."""
         self.ctx.call(f"apda_analyze_{dtype}_dev", _p(d_samples), n_samples, ld or n_samples, batch, n_fft, center,
                       int(bool(flexible)), float(fs), _p(d_fs), k, rec_cap, _p(d_spec_ws), _p(d_rec))
+        if resolve_ties and dtype == "f32":
+            self.resolve_fp32_ties_device(d_samples, batch, n_samples, n_fft, fs, d_rec, flexible, k, rec_cap, center,
+                                          d_fs, 0, ld)
+
+    def resolve_fp32_ties_device(self, d_samples: int, batch: int, n_samples: int, n_fft: int, fs: float, d_rec: int,
+                                 flexible: bool = True, k: int = 4, rec_cap: int = 5, center: int = _cabi.CENTER_MEDIAN,
+                                 d_fs: int = 0, d_n_valid: int = 0, ld: int | None = None) -> None:
+        """Replace the records (written by any fp32 picker route for these float32 samples) whose status is exactly
+        APDA_STATUS_FP32_TIE with the fp64 path's records of the widened samples; no host synchronisation."""
+        self.ctx.call("apda_resolve_fp32_ties_dev", _p(d_samples), _p(d_n_valid), n_samples, ld or n_samples, batch, n_fft,
+                      center, int(bool(flexible)), float(fs), _p(d_fs), k, rec_cap, _p(d_rec))
 
     def synth_device(self, first_window: int, count: int, n: int, dtype: str, d_out: int, seed: int = 42,
                      on_bin: bool = False) -> None:

@@ -28,7 +28,7 @@ int apda_cuda_fail(cudaError_t e, const char *what) {
     return APDA_ERR_CUDA;
 }
 extern "C" const char *apda_last_error(void) { return g_err; }
-extern "C" int apda_version(void) { return 100; }
+extern "C" int apda_version(void) { return 101; }
 
 int apda_reserve(void **buf, size_t *have, size_t need) {
     if (need <= *have) return APDA_OK;
@@ -86,6 +86,10 @@ int apda_repair_list(apda_ctx *ctx, cudaStream_t st, int64_t batch, int **out) {
 int apda_ragged_list(apda_ctx *ctx, cudaStream_t st, int64_t batch, int **out) {
     auto &l = ctx->stream_lists[st];
     return stream_list(st, &l.ragged, &l.ragged_bytes, batch, out);
+}
+int apda_tie_list(apda_ctx *ctx, cudaStream_t st, int64_t batch, int **out) {
+    auto &l = ctx->stream_lists[st];
+    return stream_list(st, &l.ties, &l.ties_bytes, batch, out);
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -145,6 +149,7 @@ extern "C" int apda_ctx_destroy(apda_ctx *ctx) {
     for (auto &kv : ctx->stream_lists) {
         cudaFree(kv.second.repair);
         cudaFree(kv.second.ragged);
+        cudaFree(kv.second.ties);
     }
     for (auto &kv : ctx->stream_scratch) cudaFree(kv.second.first);
     for (int i = 0; i < 2; ++i) {
@@ -784,6 +789,131 @@ extern "C" int apda_analyze_fused_f32_host(apda_ctx *ctx, const float *h_samples
     APDA_TRY(check_fused_args(N, flags, k, rec_cap));
     return host_pipeline<float>(ctx, kFused, h_samples, n_samples, ld, batch, N, flags, flexible, fs, h_fs, k, rec_cap, false,
                                 nullptr, h_rec);
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// fp32 tie resolution: records with status exactly APDA_STATUS_FP32_TIE get the fp64 path's record of the widened samples
+// ---------------------------------------------------------------------------------------------------------------
+static int check_resolve_args(apda_ctx *ctx, const float *samples, int64_t n_samples, int64_t ld, int64_t batch, int64_t N,
+                              int flags, int k, int rec_cap, const void *rec) {
+    APDA_TRY(check_fft_args(ctx, samples, n_samples, ld, batch, N, flags, rec));
+    return check_peaks_args(ctx, samples, N, batch, k, rec_cap, rec);
+}
+// the fp64 reference centres with the exact median; APDA_CENTER_MEAN (full-length windows only) is its fp32 shortcut
+static int resolve_center(int flags) { return flags == APDA_CENTER_MEAN ? APDA_CENTER_MEDIAN : flags; }
+
+extern "C" int apda_resolve_fp32_ties_dev(apda_ctx *ctx, const float *d_samples, const int32_t *d_n_valid,
+                                          int64_t n_samples, int64_t ld, int64_t batch, int64_t N, int flags, int flexible,
+                                          double fs, const double *d_fs, int k, int rec_cap, void *d_rec) {
+    APDA_TRY(check_resolve_args(ctx, d_samples, n_samples, ld, batch, N, flags, k, rec_cap, d_rec));
+    APDA_CUDA(cudaSetDevice(ctx->device));
+    if (N > fft_smem_max_n<double>(ctx)) {
+        apda_set_error("resolve_fp32_ties_dev: N=%lld > %lld does not fit one CTA in fp64 (use apda_resolve_fp32_ties_host)",
+                       (long long)N, (long long)fft_smem_max_n<double>(ctx));
+        return APDA_ERR_UNSUPPORTED;
+    }
+    if (batch == 0) return APDA_OK;
+    const size_t slots = resolve_ties_slot_bytes(ctx, N, batch);
+    if (slots > ctx->ws_bytes) {
+        APDA_CUDA(cudaStreamSynchronize(ctx->stream));  // old workspace may be in use
+        APDA_TRY(apda_reserve(&ctx->ws, &ctx->ws_bytes, slots));
+    }
+    int *list = nullptr;
+    APDA_TRY(apda_tie_list(ctx, ctx->stream, batch, &list));
+    return launch_resolve_ties(ctx, ctx->stream, d_samples, d_n_valid, n_samples, ld, batch, N, resolve_center(flags), flexible,
+                               fs, d_fs, k, rec_cap, d_rec, list, ctx->ws);
+}
+
+extern "C" int apda_resolve_fp32_ties_host(apda_ctx *ctx, const float *h_samples, const int32_t *h_n_valid,
+                                           int64_t n_samples, int64_t ld, int64_t batch, int64_t N, int flags, int flexible,
+                                           double fs, const double *h_fs, int k, int rec_cap, void *h_rec) {
+    APDA_TRY(check_resolve_args(ctx, h_samples, n_samples, ld, batch, N, flags, k, rec_cap, h_rec));
+    APDA_CUDA(cudaSetDevice(ctx->device));
+    const bool on_device = N <= fft_smem_max_n<double>(ctx);
+    if (!on_device && h_n_valid) {
+        apda_set_error("ragged batches are offered for N <= %lld", (long long)fft_smem_max_n<double>(ctx));
+        return APDA_ERR_UNSUPPORTED;
+    }
+    const int center = resolve_center(flags);
+    const size_t rec_bytes = (size_t)APDA_REC_BYTES(rec_cap);
+    unsigned char *recs = reinterpret_cast<unsigned char *>(h_rec);
+    std::vector<int64_t> tied;
+    for (int64_t w = 0; w < batch; ++w) {
+        int32_t status;
+        memcpy(&status, recs + (size_t)w * rec_bytes + 4, sizeof(status));
+        if (status == APDA_STATUS_FP32_TIE) tied.push_back(w);
+    }
+    const int64_t cnt = (int64_t)tied.size();
+    if (cnt == 0) return APDA_OK;
+
+    if (!on_device) {  // the fp64 analysis pipeline on the gathered, widened windows
+        std::vector<double> x((size_t)cnt * (size_t)n_samples), f(h_fs ? (size_t)cnt : 0);
+        std::vector<unsigned char> r((size_t)cnt * rec_bytes);
+        for (int64_t i = 0; i < cnt; ++i) {
+            const float *src = h_samples + (size_t)tied[(size_t)i] * (size_t)ld;
+            std::copy(src, src + n_samples, x.begin() + (size_t)i * (size_t)n_samples);
+            if (h_fs) f[(size_t)i] = h_fs[tied[(size_t)i]];
+        }
+        APDA_TRY(host_pipeline<double>(ctx, kAnalyze, x.data(), n_samples, n_samples, cnt, N, center, flexible, fs,
+                                       h_fs ? f.data() : nullptr, k, rec_cap, false, nullptr, r.data()));
+        for (int64_t i = 0; i < cnt; ++i)
+            memcpy(recs + (size_t)tied[(size_t)i] * rec_bytes, r.data() + (size_t)i * rec_bytes, rec_bytes);
+        return APDA_OK;
+    }
+
+    // the device resolver on the gathered windows (every uploaded record is tied, so every one is listed), in chunks of
+    // about 96 MB of samples on the first pipeline stream
+    int64_t chunk = std::max<int64_t>(1, (int64_t)((96u << 20) / ((size_t)n_samples * sizeof(float))));
+    chunk = std::min<int64_t>(chunk, cnt);
+    const size_t in_b = align256((size_t)chunk * (size_t)n_samples * sizeof(float)), rec_b = align256((size_t)chunk * rec_bytes);
+    const size_t fs_b = h_fs ? align256((size_t)chunk * sizeof(double)) : 0, nv_b = h_n_valid ? align256((size_t)chunk * sizeof(int)) : 0;
+    const size_t total = in_b + rec_b + fs_b + nv_b + resolve_ties_slot_bytes(ctx, N, chunk);
+    cudaStream_t st = ctx->pipe[0];
+    if (total > ctx->ws_pipe_bytes[0]) {
+        APDA_CUDA(cudaStreamSynchronize(st));
+        APDA_TRY(apda_reserve(&ctx->ws_pipe[0], &ctx->ws_pipe_bytes[0], total));
+    }
+    char *base = (char *)ctx->ws_pipe[0];
+    float *d_in = (float *)base;
+    unsigned char *d_rec = (unsigned char *)(base + in_b);
+    double *d_fs = h_fs ? (double *)(base + in_b + rec_b) : nullptr;
+    int *d_nv = h_n_valid ? (int *)(base + in_b + rec_b + fs_b) : nullptr;
+    void *d_slots = base + in_b + rec_b + fs_b + nv_b;
+    std::vector<float> x((size_t)chunk * (size_t)n_samples);
+    std::vector<unsigned char> r((size_t)chunk * rec_bytes);
+    std::vector<double> f(h_fs ? (size_t)chunk : 0);
+    std::vector<int> nv(h_n_valid ? (size_t)chunk : 0);
+    // one chunk; an error returns from the lambda only, so the stream is always drained before the host buffers go
+    auto run_chunk = [&](int64_t done, int64_t c) -> int {
+        for (int64_t i = 0; i < c; ++i) {
+            const int64_t w = tied[(size_t)(done + i)];
+            const float *src = h_samples + (size_t)w * (size_t)ld;
+            std::copy(src, src + n_samples, x.begin() + (size_t)i * (size_t)n_samples);
+            memcpy(r.data() + (size_t)i * rec_bytes, recs + (size_t)w * rec_bytes, rec_bytes);
+            if (h_fs) f[(size_t)i] = h_fs[w];
+            if (h_n_valid) nv[(size_t)i] = h_n_valid[w];
+        }
+        APDA_CUDA(cudaMemcpyAsync(d_in, x.data(), (size_t)c * (size_t)n_samples * sizeof(float), cudaMemcpyHostToDevice, st));
+        APDA_CUDA(cudaMemcpyAsync(d_rec, r.data(), (size_t)c * rec_bytes, cudaMemcpyHostToDevice, st));
+        if (d_fs) APDA_CUDA(cudaMemcpyAsync(d_fs, f.data(), (size_t)c * sizeof(double), cudaMemcpyHostToDevice, st));
+        if (d_nv) APDA_CUDA(cudaMemcpyAsync(d_nv, nv.data(), (size_t)c * sizeof(int), cudaMemcpyHostToDevice, st));
+        int *list = nullptr;
+        APDA_TRY(apda_tie_list(ctx, st, c, &list));
+        APDA_TRY(launch_resolve_ties(ctx, st, d_in, d_nv, n_samples, n_samples, c, N, center, flexible, fs, d_fs, k, rec_cap,
+                                     d_rec, list, d_slots));
+        APDA_CUDA(cudaMemcpyAsync(r.data(), d_rec, (size_t)c * rec_bytes, cudaMemcpyDeviceToHost, st));
+        return APDA_OK;
+    };
+    for (int64_t done = 0; done < cnt; done += chunk) {
+        const int64_t c = std::min<int64_t>(chunk, cnt - done);
+        const int status = run_chunk(done, c);
+        const cudaError_t e = cudaStreamSynchronize(st);
+        if (status != APDA_OK) return status;
+        if (e != cudaSuccess) return apda_cuda_fail(e, "resolve_fp32_ties_host");
+        for (int64_t i = 0; i < c; ++i)
+            memcpy(recs + (size_t)tied[(size_t)(done + i)] * rec_bytes, r.data() + (size_t)i * rec_bytes, rec_bytes);
+    }
+    return APDA_OK;
 }
 
 // ---------------------------------------------------------------------------------------------------------------

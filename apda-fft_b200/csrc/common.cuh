@@ -45,6 +45,8 @@ struct apda_ctx {
         size_t ragged_bytes = 0;
         int *repair = nullptr;  // K3 fast path: windows handed over to the general kernel
         size_t repair_bytes = 0;
+        int *ties = nullptr;  // fp32 tie resolver: windows whose record status is APDA_STATUS_FP32_TIE
+        size_t ties_bytes = 0;
     };
     std::map<cudaStream_t, StreamLists> stream_lists;
     int generic_only = 0;  // debug/test switch: bypass the specialised fp32 kernels
@@ -99,6 +101,7 @@ int apda_func_smem(const void *kernel, int device, size_t bytes);
 // per-stream window lists of `batch + 1` ints, zero count enqueued on `st` (see apda_ctx::stream_lists)
 int apda_repair_list(apda_ctx *ctx, cudaStream_t st, int64_t batch, int **out);
 int apda_ragged_list(apda_ctx *ctx, cudaStream_t st, int64_t batch, int **out);
+int apda_tie_list(apda_ctx *ctx, cudaStream_t st, int64_t batch, int **out);
 
 static inline int ilog2_i64(int64_t v) {
     int l = 0;
@@ -158,6 +161,11 @@ int launch_peaks_f32_fast(apda_ctx *ctx, cudaStream_t st, const float *d_spec, i
 int launch_center_f64(apda_ctx *ctx, cudaStream_t st, const double *d_in, int64_t n, double *d_out);
 int launch_mag_helpers_f64(apda_ctx *ctx, cudaStream_t st, const double *d_mags, int64_t n, int64_t idx, double prom_in,
                            double *d_out3);
+// fp32 tie resolver (resolve_ties.cu): d_slots holds resolve_ties_slot_bytes(ctx, N, batch) bytes of spectrum slots
+size_t resolve_ties_slot_bytes(apda_ctx *ctx, int64_t N, int64_t batch);
+int launch_resolve_ties(apda_ctx *ctx, cudaStream_t st, const float *d_samples, const int *d_nv, int64_t n_samples,
+                        int64_t ld, int64_t batch, int64_t N, int center, int flexible, double fs, const double *d_fs,
+                        int k, int rec_cap, void *d_rec, int *d_list, void *d_slots);
 
 // ---------------------------------------------------------------------------------------------------------------
 // device side

@@ -60,8 +60,9 @@ typedef struct apda_peak_rec {
 #define APDA_STATUS_EMPTY 8         /* ragged batch: empty window (the reference's pickers raise StatisticsError) */
 #define APDA_STATUS_FP32_TIE 16     /* fp32 pickers (N <= 2^15): two adjacent bins above the threshold are equal in fp32 and form
                                      * the top of a peak; the strict local-maximum test reports no peak there, the fp64
-                                     * reference (whose magnitudes differ below fp32 resolution) reports one: re-run the
-                                     * window through the fp64 entry points (apda-fft_b200/batch.py does) */
+                                     * reference (whose magnitudes differ below fp32 resolution) reports one.
+                                     * apda_resolve_fp32_ties_{dev,host} replace such records by the fp64 path's.  Plateaus
+                                     * of three or more equal bins are not flagged, so they are not resolved either. */
 #define APDA_REC_BYTES(rec_cap) (8 + 24 * (int64_t)(rec_cap))
 #define APDA_MAX_REC_CAP 64
 /* Most peaks one window of n bins can report (candidates are strict local maxima above mean + 2 sigma of the half
@@ -220,6 +221,32 @@ int apda_analyze_fused_f32_dev(apda_ctx *ctx, const float *d_samples, int64_t n_
 int apda_analyze_fused_f32_host(apda_ctx *ctx, const float *h_samples, int64_t n_samples, int64_t ld, int64_t batch,
                                 int64_t N, int flags, int flexible, double fs, const double *h_fs, int k, int rec_cap,
                                 void *h_rec);
+
+/* ---- fp32 tie resolution -----------------------------------------------------------------------------------------
+ * Replace the record of every window whose status is exactly APDA_STATUS_FP32_TIE with the record the fp64 path computes
+ * from the same samples widened to double; the records are a table written by any fp32 picker route (apda_analyze_f32_*,
+ * apda_analyze_ragged_f32_dev, apda_analyze_fused_f32_*, or apda_fft_f32_* followed by apda_peaks_*_f32_*) for these
+ * samples and these arguments.
+ *   - Only status == 16 is re-run.  A record with 16 together with other bits (e.g. APDA_STATUS_OTHER_LENGTH) keeps every
+ *     byte, and so does every other record.  Samples are read-only; no byte outside the replaced records is written.
+ *   - The new record is byte-equal to what apda_analyze_f64_dev (apda_analyze_ragged_f64_dev when n_valid is given)
+ *     writes for that window's samples widened to double, with the same n_samples, ld, N, k, rec_cap and flexible, and
+ *     fs = d_fs ? d_fs[w] : fs.
+ *   - APDA_CENTER_MEDIAN and APDA_CENTER_NONE are passed through; APDA_CENTER_MEAN (legal only at n_samples == N) becomes
+ *     APDA_CENTER_MEDIAN, the reference's centring.
+ *   - _dev enqueues on the context stream and does not synchronise the host (except when it grows its workspace, as the
+ *     other _dev calls do); it serves N <= 8192 on a B200 and returns APDA_ERR_UNSUPPORTED above.  d_rec may be a peer
+ *     table slice: call it after the picker and before apda_peer_signal.
+ *   - _host covers every N the fp64 analysis supports (ragged batches: N <= 8192): it scans h_rec, uploads only the
+ *     flagged rows, resolves them and writes their records back.
+ * Not covered: the wire-16 and text ingest (there the reference's samples are the fp64 decode, not the fp32 values: use
+ * their _f64 entry points), and the apda_peaks_* entry points (no samples). */
+int apda_resolve_fp32_ties_dev(apda_ctx *ctx, const float *d_samples, const int32_t *d_n_valid /* NULL: n_samples */,
+                               int64_t n_samples, int64_t ld, int64_t batch, int64_t N, int flags, int flexible,
+                               double fs, const double *d_fs, int k, int rec_cap, void *d_rec);
+int apda_resolve_fp32_ties_host(apda_ctx *ctx, const float *h_samples, const int32_t *h_n_valid,
+                                int64_t n_samples, int64_t ld, int64_t batch, int64_t N, int flags, int flexible,
+                                double fs, const double *h_fs, int k, int rec_cap, void *h_rec);
 
 /* ---- picker helpers on a magnitude array (module-public functions of the reference) --------------------------
  * utils/get_peak_prominence.py:32-54 calculate_prominence(magnitudes, peak_idx) */
