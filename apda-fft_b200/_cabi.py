@@ -65,6 +65,8 @@ SIGNATURES = {
     "apda_parse_samples_f64_host": (_int, [_p, _p, _p, _i64, _i64, _p, _p, _p]),
     "apda_analyze_text_f64_host": (_int, [_p, _p, _p, _i64, _i64, _i64, _int, _int, _dbl, _p, _int, _int, _p, _p, _p]),
     "apda_analyze_text_f32_host": (_int, [_p, _p, _p, _i64, _i64, _i64, _int, _int, _dbl, _p, _int, _int, _p, _p, _p]),
+    "apda_analyze_logs_f64_host": (_int, [_p, _p, _i64, _i64, _int, _int, _int, _int, _p, _p, _p, _p, _p]),
+    "apda_analyze_logs_f32_host": (_int, [_p, _p, _i64, _i64, _int, _int, _int, _int, _p, _p, _p, _p, _p]),
     "apda_analyze_fused_f32_dev": (_int, [_p, _p, _i64, _i64, _i64, _i64, _int, _int, _dbl, _p, _int, _int, _p]),
     "apda_analyze_fused_f32_host": (_int, [_p, _p, _i64, _i64, _i64, _i64, _int, _int, _dbl, _p, _int, _int, _p]),
     "apda_resolve_fp32_ties_dev": (_int, [_p, _p, _p, _i64, _i64, _i64, _i64, _int, _int, _dbl, _p, _int, _int, _p]),
@@ -90,6 +92,10 @@ def max_peaks(n: int) -> int:
 
 # record status bits (include/apda_b200.h)
 STATUS_TRUNCATED, STATUS_OTHER_LENGTH, STATUS_EMPTY, STATUS_FP32_TIE = 1, 4, 8, 16
+
+# apda_analyze_logs_*_host: header bytes per file and the per-file flag bits
+LOG_HEAD_BYTES = 1024
+LOG_SAMPLE_UNDECIDED, LOG_TOO_LONG, LOG_NO_SAMPLE_LINE, LOG_HEADER_UNDECIDED, LOG_UNREADABLE = 1, 2, 4, 8, 16
 
 
 def check_record_status(recs) -> None:

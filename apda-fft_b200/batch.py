@@ -157,6 +157,74 @@ class Analyzer:
             _cabi.check_record_status(recs)
         return recs
 
+    # ---- whole sensor .log files ----------------------------------------------------------------------------------
+    def analyze_logs(self, paths, n_fft: int, flexible: bool = True, k: int | None = None, dtype: str = "f64",
+                     strict: bool = False) -> tuple[np.ndarray, list]:
+        """Sensor ``.log`` paths -> (records[B], metas[B]): for every file what ``load_sensor`` followed by ``start_fft`` and
+        the picker computes at length ``n_fft`` with the file's own sampling rate (apda_analyze_logs_*_host: the host
+        only reads the files; headers, rates and samples are decoded on the device).  ``metas[b]`` is ``{"metadata",
+        "summary"}`` as ``load_sensor`` returns them, or None where it returns None.  Files the device leaves undecided
+        are re-read with ``load_sensor`` (so its exceptions, e.g. the ``OSError`` of ``open()``, propagate) and analysed
+        with ``analyze`` at ``n_fft``.  As on every ragged path, a file whose samples pad to another length carries
+        APDA_STATUS_OTHER_LENGTH, one without samples APDA_STATUS_EMPTY; with more than ``n_fft`` samples the record is
+        empty with APDA_STATUS_OTHER_LENGTH, and without a fifth line (meta None) empty with APDA_STATUS_EMPTY.
+        ``strict=True`` raises on any non-zero record status.  Use "f64" where the reference's samples matter (fp32
+        records are not tie-resolved)."""
+        import io
+        import os
+        from .utils import load_data
+        if dtype not in ("f64", "f32"):
+            raise ValueError(f"dtype must be 'f64' or 'f32', not {dtype!r}")
+        paths = [os.fspath(p) for p in paths]
+        b = len(paths)
+        n = int(n_fft)
+        k = (4 if flexible else 5) if k is None else int(k)
+        cap = max(5, k)
+        recs = np.zeros(b, dtype=record_dtype(cap))
+        fs = np.zeros(b, dtype=np.float64)
+        nv = np.zeros(b, dtype=np.int32)
+        fl = np.zeros(b, dtype=np.int32)
+        head = np.zeros((b, _cabi.LOG_HEAD_BYTES), dtype=np.uint8)
+        c_paths = (ctypes.c_char_p * max(b, 1))(*[os.fsencode(p) for p in paths])
+        self.ctx.call(f"apda_analyze_logs_{dtype}_host", ctypes.cast(c_paths, _p), b, n, _cabi.CENTER_MEDIAN,
+                      int(bool(flexible)), k, cap, _p(recs.ctypes.data), _p(fs.ctypes.data), _p(nv.ctypes.data),
+                      _p(fl.ctypes.data), _p(head.ctypes.data))
+        metas: list = [None] * b
+        redo = []
+        for i in range(b):
+            f = int(fl[i])
+            if f & (_cabi.LOG_SAMPLE_UNDECIDED | _cabi.LOG_HEADER_UNDECIDED | _cabi.LOG_UNREADABLE):
+                redo.append(i)
+                continue
+            if f & _cabi.LOG_NO_SAMPLE_LINE:
+                continue
+            text = head[i].tobytes().split(b"\0", 1)[0].decode("ascii")
+            try:
+                metadata, summary = load_data._parse_header(io.StringIO(text, newline=None).readlines())
+            except (ValueError, IndexError):      # load_sensor raises the same: take its route below
+                redo.append(i)
+                continue
+            metas[i] = {"metadata": metadata, "summary": summary}
+        for i in redo:
+            got = load_data.load_sensor(paths[i])
+            if got is None:
+                _empty_record(recs, i, _cabi.STATUS_EMPTY)
+                continue
+            metas[i] = {"metadata": got["metadata"], "summary": got["summary"]}
+            x = np.asarray(got["samples"], dtype=np.float64 if dtype == "f64" else np.float32)
+            if x.size > n:
+                _empty_record(recs, i, _cabi.STATUS_OTHER_LENGTH)
+            elif x.size == 0:
+                _empty_record(recs, i, _cabi.STATUS_EMPTY)
+            else:
+                recs[i] = self.analyze(x[None, :], got["metadata"]["fs"], flexible=flexible, k=k, n_fft=n, rec_cap=cap,
+                                       resolve_ties=False)[0]
+                if next_pow2(x.size) != n:
+                    recs["status"][i] |= _cabi.STATUS_OTHER_LENGTH
+        if strict:
+            _cabi.check_record_status(recs)
+        return recs, metas
+
     def analyze_host_ptr(self, h_ptr: int, batch: int, n_samples: int, n_fft: int, dtype: str, fs: float,
                          h_rec_ptr: int, flexible: bool = True, k: int = 4, rec_cap: int = 5,
                          center: int = _cabi.CENTER_MEDIAN) -> None:
@@ -214,6 +282,17 @@ class Analyzer:
         if arr.shape != (batch,):
             raise ValueError(f"fs must be a scalar or have shape ({batch},)")
         return float(arr[0]) if batch else 0.0, arr
+
+
+def _empty_record(recs: np.ndarray, i: int, status: int) -> None:
+    """The record the device writes for a window with no analysis result: count 0, every slot idx -1 and zeros."""
+    recs["count"][i] = 0
+    recs["status"][i] = status
+    pk = recs["pk"]
+    pk["idx"][i] = -1
+    pk["width_bins"][i] = 0
+    pk["mag"][i] = 0.0
+    pk["prominence"][i] = 0.0
 
 
 def multi_analyze(contexts, samples: np.ndarray, fs, flexible: bool = True, k: int | None = None,

@@ -1,10 +1,16 @@
 // C ABI of libapda_b200.so (declared in include/apda_b200.h): context, twiddle tables, dispatch, host pipelines.
+#include <errno.h>
+#include <fcntl.h>
 #include <math.h>
 #include <stdarg.h>
 #include <stdio.h>
 #include <string.h>
+#include <sys/stat.h>
+#include <unistd.h>
 
 #include <algorithm>
+#include <atomic>
+#include <functional>
 #include <mutex>
 #include <string>
 #include <thread>
@@ -28,7 +34,7 @@ int apda_cuda_fail(cudaError_t e, const char *what) {
     return APDA_ERR_CUDA;
 }
 extern "C" const char *apda_last_error(void) { return g_err; }
-extern "C" int apda_version(void) { return 101; }
+extern "C" int apda_version(void) { return 102; }
 
 int apda_reserve(void **buf, size_t *have, size_t need) {
     if (need <= *have) return APDA_OK;
@@ -154,6 +160,7 @@ extern "C" int apda_ctx_destroy(apda_ctx *ctx) {
     for (auto &kv : ctx->stream_scratch) cudaFree(kv.second.first);
     for (int i = 0; i < 2; ++i) {
         cudaFree(ctx->ws_pipe[i]);
+        cudaFreeHost(ctx->log_stage[i]);
         if (ctx->pipe[i]) cudaStreamDestroy(ctx->pipe[i]);
     }
     if (ctx->own_stream) cudaStreamDestroy(ctx->own_stream);
@@ -1179,6 +1186,257 @@ extern "C" int apda_analyze_text_f32_host(apda_ctx *ctx, const char *h_text, con
                                           int32_t *h_flags) {
     return analyze_text_host<float>(ctx, h_text, h_offsets, batch, n_max, N, flags, flexible, fs, h_fs, k, rec_cap, h_rec,
                                     h_n_valid, h_flags);
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// whole sensor logs: paths -> file bytes in pinned staging (reader threads) -> header layout, samples, records on the
+// device.  The host never looks inside a file.
+// ---------------------------------------------------------------------------------------------------------------
+namespace {
+
+// Fork-join reader threads: run(n, fn) calls fn(0 .. n-1) on min(16, hardware threads, n) threads and returns at
+// once; join() (also run by the destructor, so every error path joins) waits for them.  A thread that cannot be
+// created leaves its share to the others; with none at all the caller's thread does the work inside run().
+class ReaderThreads {
+   public:
+    ~ReaderThreads() { join(); }
+    void run(int64_t n, std::function<void(int64_t)> fn) {
+        join();
+        next_ = 0;
+        n_ = n;
+        fn_ = std::move(fn);
+        const unsigned hw = std::thread::hardware_concurrency();
+        const int64_t want = std::min<int64_t>(n, std::min(16u, hw ? hw : 1u));
+        for (int64_t i = 0; i < want; ++i) {
+            try {
+                threads_.emplace_back([this] { work(); });
+            } catch (...) {
+                break;
+            }
+        }
+        if (threads_.empty()) work();
+    }
+    void join() {
+        for (auto &t : threads_) t.join();
+        threads_.clear();
+    }
+
+   private:
+    void work() {
+        for (int64_t i; (i = next_.fetch_add(1)) < n_;) fn_(i);
+    }
+    std::atomic<int64_t> next_{0};
+    int64_t n_ = 0;
+    std::function<void(int64_t)> fn_;
+    std::vector<std::thread> threads_;
+};
+
+// size of a regular file, or -1 (missing, unreadable, directory, device, fifo ...)
+int64_t log_file_size(const char *path) {
+    struct stat sb;
+    if (stat(path, &sb) != 0 || !S_ISREG(sb.st_mode)) return -1;
+    return (int64_t)sb.st_size;
+}
+
+// the whole file into dst; false unless it is still a regular file of exactly `size` bytes and every byte was read
+bool read_log_file(const char *path, char *dst, int64_t size) {
+    const int fd = open(path, O_RDONLY | O_CLOEXEC | O_NONBLOCK);
+    if (fd < 0) return false;
+    struct stat sb;
+    bool ok = fstat(fd, &sb) == 0 && S_ISREG(sb.st_mode) && (int64_t)sb.st_size == size;
+    for (int64_t got = 0; ok && got < size;) {
+        const ssize_t r = pread(fd, dst + got, (size_t)(size - got), (off_t)got);
+        if (r < 0 && errno == EINTR) continue;
+        if (r <= 0) ok = false;
+        else got += r;
+    }
+    close(fd);
+    return ok;
+}
+
+int reserve_pinned(cudaStream_t user, void **buf, size_t *have, size_t need) {
+    if (need <= *have) return APDA_OK;
+    APDA_CUDA(cudaStreamSynchronize(user));  // the old buffer may still feed a copy on this stream
+    if (*buf) APDA_CUDA(cudaFreeHost(*buf));
+    *buf = nullptr;
+    *have = 0;
+    const cudaError_t e = cudaHostAlloc(buf, need, cudaHostAllocDefault);
+    if (e != cudaSuccess) {
+        *buf = nullptr;
+        apda_set_error("cudaHostAlloc(%zu) failed: %s", need, cudaGetErrorString(e));
+        (void)cudaGetLastError();
+        return APDA_ERR_NOMEM;
+    }
+    *have = need;
+    return APDA_OK;
+}
+
+}  // namespace
+
+// a chunk holds at most this many file bytes (a larger file is a chunk of its own)
+static const int64_t kLogChunkBytes = int64_t(64) << 20;
+
+template <typename T>
+static int analyze_logs_host(apda_ctx *ctx, const char *const *paths, int64_t n_files, int64_t N, int flags, int flexible,
+                             int k, int rec_cap, void *h_rec, double *h_fs, int32_t *h_n_valid, int32_t *h_flags,
+                             char *h_head) {
+    if (!ctx || !paths || !h_rec || !h_fs || !h_n_valid || !h_flags || !h_head || n_files < 0 || n_files > 0x7fffffff) {
+        apda_set_error("analyze_logs: bad arguments (NULL buffer or n_files out of range)");
+        return APDA_ERR_INVALID;
+    }
+    if (!is_pow2_i64(N) || N < 4 || N > fft_smem_max_n<T>(ctx)) {
+        apda_set_error("analyze_logs: N=%lld must be a power of two in [4, %lld]", (long long)N,
+                       (long long)fft_smem_max_n<T>(ctx));
+        return APDA_ERR_INVALID;
+    }
+    if (flags != APDA_CENTER_MEDIAN && flags != APDA_CENTER_NONE) {
+        apda_set_error("analyze_logs: flags must be APDA_CENTER_MEDIAN or APDA_CENTER_NONE");
+        return APDA_ERR_INVALID;
+    }
+    APDA_TRY(check_peaks_args(ctx, h_rec, N, n_files, k, rec_cap, h_rec));
+    for (int64_t b = 0; b < n_files; ++b)
+        if (!paths[b]) {
+            apda_set_error("analyze_logs: paths[%lld] is NULL", (long long)b);
+            return APDA_ERR_INVALID;
+        }
+    APDA_CUDA(cudaSetDevice(ctx->device));
+    if (n_files == 0) return APDA_OK;
+    const size_t rec_bytes = (size_t)APDA_REC_BYTES(rec_cap);
+
+    ReaderThreads readers;
+    std::vector<int64_t> size((size_t)n_files);
+    readers.run(n_files, [&](int64_t b) { size[(size_t)b] = log_file_size(paths[b]); });
+    readers.join();
+
+    // chunks: at most kLogChunkBytes of text and as many files as ~96 MB of spectra hold
+    const int64_t max_files = std::max<int64_t>(1, (int64_t)((96u << 20) / ((size_t)N * 2 * sizeof(T))));
+    std::vector<int64_t> first;  // first file of every chunk, then n_files
+    int64_t max_text = 0, max_cnt = 0;
+    for (int64_t b = 0, bytes = 0; b < n_files; ++b) {
+        const int64_t s = std::max<int64_t>(size[(size_t)b], 0);
+        if (first.empty() || b - first.back() == max_files || (b > first.back() && bytes + s > kLogChunkBytes)) {
+            first.push_back(b);
+            bytes = 0;
+        }
+        bytes += s;
+        max_text = std::max(max_text, bytes);
+        max_cnt = std::max(max_cnt, b - first.back() + 1);
+    }
+    first.push_back(n_files);
+    const int64_t n_chunks = (int64_t)first.size() - 1;
+
+    // device workspace of one chunk (per stream) and pinned staging: text, then the chunk-relative offsets
+    const size_t txt_b = align256((size_t)max_text + 16), off_b = align256((size_t)(max_cnt + 1) * sizeof(int64_t));
+    const size_t start_b = align256((size_t)max_cnt * sizeof(int64_t)), fs_b = align256((size_t)max_cnt * sizeof(double));
+    const size_t int_b = align256((size_t)max_cnt * sizeof(int)), head_b = align256((size_t)max_cnt * APDA_LOG_HEAD_BYTES);
+    const size_t smp_b = align256((size_t)max_cnt * (size_t)N * sizeof(T));
+    const size_t spec_b = align256((size_t)max_cnt * (size_t)N * 2 * sizeof(T)), recs_b = align256((size_t)max_cnt * rec_bytes);
+    const size_t mag_b = align256(peaks_mag_workspace_bytes<T>(ctx, N, max_cnt));
+    const size_t total = txt_b + off_b + start_b + fs_b + 3 * int_b + head_b + smp_b + spec_b + recs_b + mag_b;
+    for (int s = 0; s < 2 && s < n_chunks; ++s) {
+        if (total > ctx->ws_pipe_bytes[s]) {
+            APDA_CUDA(cudaStreamSynchronize(ctx->pipe[s]));
+            APDA_TRY(apda_reserve(&ctx->ws_pipe[s], &ctx->ws_pipe_bytes[s], total));
+        }
+        APDA_TRY(reserve_pinned(ctx->pipe[s], &ctx->log_stage[s], &ctx->log_stage_bytes[s], txt_b + off_b));
+    }
+
+    std::vector<char> unread((size_t)n_files, 0);
+    // reader threads put chunk c's files into staging buffer c & 1 (returns at once; readers.join() waits)
+    auto fill = [&](int64_t c) {
+        char *stage = (char *)ctx->log_stage[c & 1];
+        int64_t *off = (int64_t *)(stage + txt_b);
+        const int64_t lo = first[(size_t)c], cnt = first[(size_t)c + 1] - lo;
+        off[0] = 0;
+        for (int64_t i = 0; i < cnt; ++i) off[i + 1] = off[i] + std::max<int64_t>(size[(size_t)(lo + i)], 0);
+        readers.run(cnt, [&, stage, off, lo](int64_t i) {
+            const int64_t b = lo + i;
+            if (size[(size_t)b] < 0 || !read_log_file(paths[b], stage + off[i], size[(size_t)b])) unread[(size_t)b] = 1;
+        });
+    };
+    auto run_chunk = [&](int64_t c) -> int {  // see host_pipeline: errors never skip the drain
+        const int s = (int)(c & 1);
+        cudaStream_t st = ctx->pipe[s];
+        const int64_t lo = first[(size_t)c], cnt = first[(size_t)c + 1] - lo;
+        const char *stage = (const char *)ctx->log_stage[s];
+        const int64_t *off = (const int64_t *)(stage + txt_b);
+        char *p = (char *)ctx->ws_pipe[s];
+        char *d_txt = p;                   p += txt_b;
+        int64_t *d_off = (int64_t *)p;     p += off_b;
+        int64_t *d_start = (int64_t *)p;   p += start_b;
+        double *d_fs = (double *)p;        p += fs_b;
+        int *d_fl = (int *)p;              p += int_b;
+        int *d_pfl = (int *)p;             p += int_b;
+        int *d_nv = (int *)p;              p += int_b;
+        char *d_head = p;                  p += head_b;
+        T *d_smp = (T *)p;                 p += smp_b;
+        T *d_spec = (T *)p;                p += spec_b;
+        void *d_rec = p;                   p += recs_b;
+        void *mag_ws = mag_b ? (void *)p : nullptr;
+        size_t mag_have = mag_b;
+        APDA_CUDA(cudaMemcpyAsync(d_txt, stage, (size_t)off[cnt], cudaMemcpyHostToDevice, st));
+        APDA_CUDA(cudaMemcpyAsync(d_off, off, (size_t)(cnt + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, st));
+        APDA_TRY(launch_log_layout(ctx, st, d_txt, d_off, cnt, d_start, d_fs, d_fl, d_head));
+        APDA_TRY(launch_parse_samples<T>(ctx, st, d_txt, d_off, cnt, N, d_smp, d_nv, d_pfl, d_start));
+        APDA_TRY(analyze_ragged_dev<T>(ctx, st, d_smp, d_nv, N, N, cnt, N, flags, flexible, 0.0, d_fs, k, rec_cap, d_spec,
+                                       d_rec, &mag_ws, &mag_have, 0));
+        APDA_TRY(launch_log_finish(ctx, st, cnt, d_fl, d_pfl, d_rec, rec_cap));
+        APDA_CUDA(cudaMemcpyAsync((char *)h_rec + (size_t)lo * rec_bytes, d_rec, (size_t)cnt * rec_bytes,
+                                  cudaMemcpyDeviceToHost, st));
+        APDA_CUDA(cudaMemcpyAsync(h_fs + lo, d_fs, (size_t)cnt * sizeof(double), cudaMemcpyDeviceToHost, st));
+        APDA_CUDA(cudaMemcpyAsync(h_n_valid + lo, d_nv, (size_t)cnt * sizeof(int), cudaMemcpyDeviceToHost, st));
+        APDA_CUDA(cudaMemcpyAsync(h_flags + lo, d_fl, (size_t)cnt * sizeof(int), cudaMemcpyDeviceToHost, st));
+        APDA_CUDA(cudaMemcpyAsync(h_head + (size_t)lo * APDA_LOG_HEAD_BYTES, d_head, (size_t)cnt * APDA_LOG_HEAD_BYTES,
+                                  cudaMemcpyDeviceToHost, st));
+        return APDA_OK;
+    };
+    fill(0);
+    readers.join();
+    int status = APDA_OK;
+    for (int64_t c = 0; c < n_chunks && status == APDA_OK; ++c) {
+        if (c + 1 < n_chunks) {
+            // staging buffer (c + 1) & 1 fed chunk c - 1, whose copies were enqueued on the same stream
+            const cudaError_t e = cudaStreamSynchronize(ctx->pipe[(c + 1) & 1]);
+            if (e != cudaSuccess) {
+                status = apda_cuda_fail(e, "analyze_logs (staging reuse)");
+                break;
+            }
+            fill(c + 1);
+        }
+        status = run_chunk(c);
+        readers.join();
+    }
+    readers.join();
+    cudaError_t e0 = cudaStreamSynchronize(ctx->pipe[0]);
+    cudaError_t e1 = cudaStreamSynchronize(ctx->pipe[1]);
+    if (status != APDA_OK) return status;
+    if (e0 != cudaSuccess) return apda_cuda_fail(e0, "analyze_logs (stream 0)");
+    if (e1 != cudaSuccess) return apda_cuda_fail(e1, "analyze_logs (stream 1)");
+    for (int64_t b = 0; b < n_files; ++b) {
+        if (!unread[(size_t)b]) continue;
+        h_flags[b] = 16;
+        h_fs[b] = 0.0;
+        h_n_valid[b] = 0;
+        memset(h_head + (size_t)b * APDA_LOG_HEAD_BYTES, 0, APDA_LOG_HEAD_BYTES);
+        char *rec = (char *)h_rec + (size_t)b * rec_bytes;  // the empty record, status 0
+        const int32_t hdr[2] = {0, 0};
+        const apda_peak none{-1, 0, 0.0, 0.0};
+        memcpy(rec, hdr, sizeof(hdr));
+        for (int i = 0; i < rec_cap; ++i) memcpy(rec + 8 + (size_t)i * sizeof(apda_peak), &none, sizeof(none));
+    }
+    return APDA_OK;
+}
+extern "C" int apda_analyze_logs_f64_host(apda_ctx *ctx, const char *const *paths, int64_t n_files, int64_t N, int flags,
+                                          int flexible, int k, int rec_cap, void *h_rec, double *h_fs, int32_t *h_n_valid,
+                                          int32_t *h_flags, char *h_head) {
+    return analyze_logs_host<double>(ctx, paths, n_files, N, flags, flexible, k, rec_cap, h_rec, h_fs, h_n_valid, h_flags,
+                                     h_head);
+}
+extern "C" int apda_analyze_logs_f32_host(apda_ctx *ctx, const char *const *paths, int64_t n_files, int64_t N, int flags,
+                                          int flexible, int k, int rec_cap, void *h_rec, double *h_fs, int32_t *h_n_valid,
+                                          int32_t *h_flags, char *h_head) {
+    return analyze_logs_host<float>(ctx, paths, n_files, N, flags, flexible, k, rec_cap, h_rec, h_fs, h_n_valid, h_flags,
+                                    h_head);
 }
 
 // ---------------------------------------------------------------------------------------------------------------

@@ -50,6 +50,9 @@ struct apda_ctx {
     };
     std::map<cudaStream_t, StreamLists> stream_lists;
     int generic_only = 0;  // debug/test switch: bypass the specialised fp32 kernels
+    // pinned staging of apda_analyze_logs_*_host, one per pipeline stream: file bytes, then the chunk's offsets
+    void *log_stage[2] = {nullptr, nullptr};
+    size_t log_stage_bytes[2] = {0, 0};
 };
 
 void apda_set_error(const char *fmt, ...);
@@ -137,9 +140,15 @@ int launch_fused_f32(apda_ctx *ctx, cudaStream_t st, const float *d_samples, int
 template <typename T>
 int launch_decode_wire16(apda_ctx *ctx, cudaStream_t st, const unsigned char *d_payload, int64_t n_max, int64_t ld_bytes,
                          int64_t batch, const double *d_first_value, T *d_samples, int64_t ld_out, int *d_n_valid);
+// d_starts: where each log's sample region begins (NULL: at d_offsets[b]); it ends at d_offsets[b + 1]
 template <typename T>
 int launch_parse_samples(apda_ctx *ctx, cudaStream_t st, const char *d_text, const int64_t *d_offsets, int64_t batch,
-                         int64_t ld, T *d_samples, int *d_n_valid, int *d_flags);
+                         int64_t ld, T *d_samples, int *d_n_valid, int *d_flags, const int64_t *d_starts = nullptr);
+// whole .log files (text_ingest.cu): header layout, sampling rate and header bytes; then the flags / empty records
+int launch_log_layout(apda_ctx *ctx, cudaStream_t st, const char *d_text, const int64_t *d_offsets, int64_t batch,
+                      int64_t *d_starts, double *d_fs, int *d_flags, char *d_head);
+int launch_log_finish(apda_ctx *ctx, cudaStream_t st, int64_t batch, int *d_flags, const int *d_parse_flags, void *d_rec,
+                      int rec_cap);
 bool fft_f64_fast_supports(int64_t N);
 int launch_fft_f64_fast(apda_ctx *ctx, cudaStream_t st, const double *d_samples, int64_t n_samples, int64_t ld,
                         int64_t batch, int64_t N, int flags, double *d_spec, const int *d_nv = nullptr);

@@ -211,6 +211,37 @@ int apda_analyze_text_f32_host(apda_ctx *ctx, const char *h_text, const int64_t 
                                int64_t N, int flags, int flexible, double fs, const double *h_fs, int k, int rec_cap,
                                void *h_rec, int32_t *h_n_valid, int32_t *h_flags);
 
+/* ---- whole sensor logs -----------------------------------------------------------------------------------------
+ * replaces utils/load_data.py:64-70 load_sensor(path) followed by start_fft + picker (GT_FFT_v5.py:635-642) for many
+ * .log files at once.  The host only reads bytes: reader threads (min(16, hardware threads), all joined before the call
+ * returns) pread whole files into pinned staging buffers owned by the context, chunk c + 1 while the two pipeline
+ * streams process chunk c.  The header layout, the sampling rate and the samples are decoded on the device.
+ * Per file b:
+ *   h_fs[b]       rate of header line 0, float(rate.replace(" Hz", "")) (bit-equal to Python)
+ *   h_n_valid[b]  samples parsed (at most N)
+ *   h_head[b]     the bytes of the four header lines (line ends included), NUL-padded to APDA_LOG_HEAD_BYTES
+ *   h_rec[b]      the record of apda_analyze_ragged_*_dev at n_max = ld = N on the file's samples with fs = h_fs[b]
+ *                 (windows that pad to another length carry APDA_STATUS_OTHER_LENGTH, empty ones APDA_STATUS_EMPTY)
+ * h_flags[b] (a record of a file with a non-zero flag is not an analysis result: count 0, every slot idx -1 and zeros):
+ *   1   a sample piece in a float() syntax the device does not decide (exponent, '_', > 15 significant digits,
+ *       non-ASCII): status 0, re-read the file on the host
+ *   2   more than N samples: status APDA_STATUS_OTHER_LENGTH
+ *   4   fewer than 5 lines (load_sensor returns None): status APDA_STATUS_EMPTY
+ *   8   header not decided on the device (no 4th line end within APDA_LOG_HEAD_BYTES - 1 bytes, a non-ASCII or NUL byte
+ *       in it, fewer than 4 ';' fields on line 0, a rate field outside the sample grammar once " Hz" is removed):
+ *       status 0, re-read the file on the host
+ *   16  the path is not a regular file, or could not be opened or read whole: status 0
+ * With flag 4, 8 or 16 h_fs, h_n_valid and h_head are 0.  N: a power of two from 4 up to the ragged batches' limit (on a
+ * B200 8192 in fp64, 16384 in fp32); flags: APDA_CENTER_MEDIAN or APDA_CENTER_NONE.  Use _f64 where the reference's
+ * samples matter: they are the fp64 parse (fp32 records are not tie-resolved). */
+#define APDA_LOG_HEAD_BYTES 1024
+int apda_analyze_logs_f64_host(apda_ctx *ctx, const char *const *paths, int64_t n_files, int64_t N, int flags,
+                               int flexible, int k, int rec_cap, void *h_rec, double *h_fs, int32_t *h_n_valid,
+                               int32_t *h_flags, char *h_head);
+int apda_analyze_logs_f32_host(apda_ctx *ctx, const char *const *paths, int64_t n_files, int64_t N, int flags,
+                               int flexible, int k, int rec_cap, void *h_rec, double *h_fs, int32_t *h_n_valid,
+                               int32_t *h_flags, char *h_head);
+
 /* Fused window -> record kernel (fp32, N in {1024, 2048, 4096, 8192}, k <= 5, rec_cap == 5): same records as
  * apda_analyze_f32_*, but the spectrum never exists in memory (HBM traffic s*N + 128 bytes per window instead of
  * 4*s*N + 128).  A throughput variant for fleets that only need the peak tables (SURVEY.md 8f rank 1); the drop-in
