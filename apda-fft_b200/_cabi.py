@@ -71,7 +71,11 @@ SIGNATURES = {
     "apda_analyze_fused_f32_host": (_int, [_p, _p, _i64, _i64, _i64, _i64, _int, _int, _dbl, _p, _int, _int, _p]),
     "apda_resolve_fp32_ties_dev": (_int, [_p, _p, _p, _i64, _i64, _i64, _i64, _int, _int, _dbl, _p, _int, _int, _p]),
     "apda_resolve_fp32_ties_host": (_int, [_p, _p, _p, _i64, _i64, _i64, _i64, _int, _int, _dbl, _p, _int, _int, _p]),
-    "apda_prominence_f64_host": (_int, [_p, _p, _i64, _i64, _c.POINTER(_dbl)]),
+    "apda_present_dev": (_int, [_p, _p, _int, _i64, _i64, _dbl, _p, _int, _int, _p, _p, _p, _p, _p, _p]),
+    "apda_present_host": (_int, [_p, _p, _int, _i64, _i64, _dbl, _p, _int, _int, _p, _p, _p, _p, _p, _p]),
+    "apda_fleet_jsonl_dev": (_int, [_p, _p, _int, _i64, _i64, _dbl, _p, _int, _int, _i64, _p, _i64, _p]),
+    "apda_fleet_jsonl_host": (_int, [_p, _p, _int, _i64, _i64, _dbl, _p, _int, _int, _i64, _p, _i64, _p]),
+    "apda_prominence_f64_host":(_int, [_p, _p, _i64, _i64, _c.POINTER(_dbl)]),
     "apda_half_power_bins_f64_host": (_int, [_p, _p, _i64, _dbl, _i64, _c.POINTER(_i64)]),
     "apda_half_height_bins_f64_host": (_int, [_p, _p, _i64, _i64, _c.POINTER(_i64)]),
     "apda_synth_f64_dev": (_int, [_p, _i64, _i64, _i64, _u64, _int, _p]),
@@ -88,6 +92,11 @@ SIGNATURES = {
 def max_peaks(n: int) -> int:
     """include/apda_b200.h APDA_MAX_PEAKS(n): most peaks one window of n bins can report."""
     return int(n) // 8 + 8
+
+
+def jsonl_row_bytes(k: int) -> int:
+    """include/apda_b200.h APDA_JSONL_ROW_BYTES(k): bound on the bytes of one fleet JSONL row with k peaks."""
+    return 64 + 52 * int(k)
 
 
 # record status bits (include/apda_b200.h)

@@ -264,6 +264,59 @@ class Analyzer:
         self.ctx.call("apda_resolve_fp32_ties_dev", _p(d_samples), _p(d_n_valid), n_samples, ld or n_samples, batch, n_fft,
                       center, int(bool(flexible)), float(fs), _p(d_fs), k, rec_cap, _p(d_rec))
 
+    # ---- record presentation (the reference's rounded fields, fleet JSONL rows) ----------------------------------------
+    def present(self, recs: np.ndarray, fs, n: int, flexible: bool = True, k: int | None = None) -> dict:
+        """records[B] -> dict of [B, k] numpy columns ``idx``, ``freq``, ``mag`` (plus ``prominence``, ``damping``,
+        ``q_factor`` when ``flexible``): the fields of ``records.prominence_dicts`` / ``resolution_dicts`` computed on the
+        device, bit-equal; slots past a window's count hold idx -1 and NaN.  ``k`` defaults to every slot of the record."""
+        recs = np.ascontiguousarray(np.atleast_1d(recs))
+        cap = recs.dtype["pk"].shape[0]
+        k = cap if k is None else int(k)
+        b = recs.shape[0]
+        names = ["idx", "freq", "mag"] + (["prominence", "damping", "q_factor"] if flexible else [])
+        out = {name: np.empty((b, k), dtype=np.int32 if name == "idx" else np.float64) for name in names}
+        ptr = {name: _p(a.ctypes.data) for name, a in out.items()}
+        fs_scalar, fs_arr = self._fs(fs, b)
+        self.ctx.call("apda_present_host", _p(recs.ctypes.data), cap, b, int(n), fs_scalar,
+                      _p(fs_arr.ctypes.data if fs_arr is not None else 0), int(bool(flexible)), k, ptr["idx"], ptr["freq"],
+                      ptr["mag"], ptr.get("prominence", _p(0)), ptr.get("damping", _p(0)), ptr.get("q_factor", _p(0)))
+        return out
+
+    def present_device(self, d_rec: int, batch: int, rec_cap: int, n: int, fs: float, k: int, d_idx: int = 0,
+                       d_freq: int = 0, d_mag: int = 0, d_prominence: int = 0, d_damping: int = 0, d_q: int = 0,
+                       flexible: bool = True, d_fs: int = 0) -> None:
+        """``present`` on device buffers ([batch, k] columns; 0 = not written); no host synchronisation."""
+        self.ctx.call("apda_present_dev", _p(d_rec), rec_cap, batch, n, float(fs), _p(d_fs), int(bool(flexible)), k,
+                      _p(d_idx), _p(d_freq), _p(d_mag), _p(d_prominence), _p(d_damping), _p(d_q))
+
+    def fleet_jsonl(self, recs: np.ndarray, fs, n: int, flexible: bool = True, k: int = 4, first_window: int = 0,
+                    path=None):
+        """The text ``records.write_fleet_jsonl`` writes, byte for byte, made on the device: the bytes, or (``path``
+        given) the number of rows written to that file."""
+        recs = np.ascontiguousarray(np.atleast_1d(recs))
+        cap = recs.dtype["pk"].shape[0]
+        b = recs.shape[0]
+        fs_scalar, fs_arr = self._fs(fs, b)
+        text = np.empty(max(1, b * _cabi.jsonl_row_bytes(k)), dtype=np.uint8)
+        offsets = np.empty(b + 1, dtype=np.int64)
+        self.ctx.call("apda_fleet_jsonl_host", _p(recs.ctypes.data), cap, b, int(n), fs_scalar,
+                      _p(fs_arr.ctypes.data if fs_arr is not None else 0), int(bool(flexible)), int(k), int(first_window),
+                      _p(text.ctypes.data), text.size, _p(offsets.ctypes.data))
+        rows = memoryview(text)[:int(offsets[b])]
+        if path is None:
+            return bytes(rows)
+        with open(path, "wb") as fh:
+            fh.write(rows)
+        return b
+
+    def fleet_jsonl_device(self, d_rec: int, batch: int, rec_cap: int, n: int, fs: float, d_text: int, text_cap: int,
+                           d_offsets: int, flexible: bool = True, k: int = 4, first_window: int = 0,
+                           d_fs: int = 0) -> None:
+        """``fleet_jsonl`` into device buffers: ``text_cap >= batch * _cabi.jsonl_row_bytes(k)`` bytes of text and
+        ``batch + 1`` int64 offsets (row w is text[offsets[w]:offsets[w + 1]]); no host synchronisation."""
+        self.ctx.call("apda_fleet_jsonl_dev", _p(d_rec), rec_cap, batch, n, float(fs), _p(d_fs), int(bool(flexible)), k,
+                      first_window, _p(d_text), text_cap, _p(d_offsets))
+
     def synth_device(self, first_window: int, count: int, n: int, dtype: str, d_out: int, seed: int = 42,
                      on_bin: bool = False) -> None:
         self.ctx.call(f"apda_synth_{dtype}_dev", first_window, count, n, seed, int(on_bin), _p(d_out))

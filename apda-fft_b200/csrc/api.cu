@@ -34,7 +34,7 @@ int apda_cuda_fail(cudaError_t e, const char *what) {
     return APDA_ERR_CUDA;
 }
 extern "C" const char *apda_last_error(void) { return g_err; }
-extern "C" int apda_version(void) { return 102; }
+extern "C" int apda_version(void) { return 103; }
 
 int apda_reserve(void **buf, size_t *have, size_t need) {
     if (need <= *have) return APDA_OK;
@@ -156,6 +156,7 @@ extern "C" int apda_ctx_destroy(apda_ctx *ctx) {
         cudaFree(kv.second.repair);
         cudaFree(kv.second.ragged);
         cudaFree(kv.second.ties);
+        cudaFree(kv.second.jsonl);
     }
     for (auto &kv : ctx->stream_scratch) cudaFree(kv.second.first);
     for (int i = 0; i < 2; ++i) {
@@ -1437,6 +1438,208 @@ extern "C" int apda_analyze_logs_f32_host(apda_ctx *ctx, const char *const *path
                                           int32_t *h_flags, char *h_head) {
     return analyze_logs_host<float>(ctx, paths, n_files, N, flags, flexible, k, rec_cap, h_rec, h_fs, h_n_valid, h_flags,
                                     h_head);
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// record presentation: the reference's rounded peak fields and the fleet JSONL rows, computed on the device
+// ---------------------------------------------------------------------------------------------------------------
+static int check_present_args(apda_ctx *ctx, const void *rec, int rec_cap, int64_t batch, int64_t n, int k,
+                              int64_t first_window) {
+    if (!ctx || !rec) {
+        apda_set_error("present: NULL context or records");
+        return APDA_ERR_INVALID;
+    }
+    if ((uintptr_t)rec % 8) {
+        apda_set_error("present: records must be 8-byte aligned");
+        return APDA_ERR_INVALID;
+    }
+    if (!is_pow2_i64(n) || n < 4 || n > (int64_t(1) << 30)) {
+        apda_set_error("present: n=%lld must be a power of two in [4, 2^30]", (long long)n);
+        return APDA_ERR_INVALID;
+    }
+    if (rec_cap < 1 || (rec_cap > APDA_MAX_REC_CAP && (int64_t)rec_cap > APDA_MAX_PEAKS(n))) {
+        apda_set_error("present: need 1 <= rec_cap (%d) <= max(%d, n/8 + 8 = %lld)", rec_cap, APDA_MAX_REC_CAP,
+                       (long long)APDA_MAX_PEAKS(n));
+        return APDA_ERR_INVALID;
+    }
+    if (k < 1 || k > rec_cap) {
+        apda_set_error("present: need 1 <= k (%d) <= rec_cap (%d)", k, rec_cap);
+        return APDA_ERR_INVALID;
+    }
+    if (batch < 0 || batch > 0x7fffffff) {
+        apda_set_error("present: batch %lld out of range", (long long)batch);
+        return APDA_ERR_INVALID;
+    }
+    if (first_window < 0 || first_window > INT64_MAX - batch) {
+        apda_set_error("present: first_window %lld must be >= 0 and first_window + batch must fit int64",
+                       (long long)first_window);
+        return APDA_ERR_INVALID;
+    }
+    return APDA_OK;
+}
+
+extern "C" int apda_present_dev(apda_ctx *ctx, const void *d_rec, int rec_cap, int64_t batch, int64_t n, double fs,
+                                const double *d_fs, int flexible, int k, int32_t *d_idx, double *d_freq, double *d_mag,
+                                double *d_prominence, double *d_damping, double *d_q) {
+    APDA_TRY(check_present_args(ctx, d_rec, rec_cap, batch, n, k, 0));
+    APDA_CUDA(cudaSetDevice(ctx->device));
+    return launch_present_columns(ctx, ctx->stream, d_rec, rec_cap, batch, n, fs, d_fs, flexible, k, d_idx, d_freq, d_mag,
+                                  d_prominence, d_damping, d_q);
+}
+
+extern "C" int apda_present_host(apda_ctx *ctx, const void *h_rec, int rec_cap, int64_t batch, int64_t n, double fs,
+                                 const double *h_fs, int flexible, int k, int32_t *h_idx, double *h_freq, double *h_mag,
+                                 double *h_prominence, double *h_damping, double *h_q) {
+    APDA_TRY(check_present_args(ctx, h_rec, rec_cap, batch, n, k, 0));
+    APDA_CUDA(cudaSetDevice(ctx->device));
+    if (batch == 0) return APDA_OK;
+    double *h_col[5] = {h_freq, h_mag, h_prominence, h_damping, h_q};
+    int ncol = 0;
+    for (double *c : h_col) ncol += c != nullptr;
+    const size_t rec_bytes = (size_t)APDA_REC_BYTES(rec_cap);
+    const size_t per_window = rec_bytes + (h_fs ? 8 : 0) + (size_t)k * ((h_idx ? 4 : 0) + 8 * ncol);
+    // chunk: ~64 MB of staging per stream, at least one window
+    int64_t chunk = std::min<int64_t>(batch, std::max<int64_t>(1, (int64_t)((64u << 20) / per_window)));
+    if (batch > chunk && batch < 2 * chunk) chunk = (batch + 1) / 2;
+    const size_t rec_b = align256((size_t)chunk * rec_bytes), fs_b = h_fs ? align256((size_t)chunk * 8) : 0;
+    const size_t idx_b = h_idx ? align256((size_t)chunk * k * 4) : 0, col_b = align256((size_t)chunk * k * 8);
+    const size_t total = rec_b + fs_b + idx_b + col_b * ncol;
+    for (int s = 0; s < 2; ++s) {
+        if (total > ctx->ws_pipe_bytes[s]) {
+            APDA_CUDA(cudaStreamSynchronize(ctx->pipe[s]));
+            APDA_TRY(apda_reserve(&ctx->ws_pipe[s], &ctx->ws_pipe_bytes[s], total));
+        }
+        if (batch <= chunk) break;
+    }
+    // an error returns from the lambda only, so both streams are drained before the caller's buffers are released
+    auto run_chunk = [&](int c, int64_t done, int64_t cnt) -> int {
+        cudaStream_t st = ctx->pipe[c & 1];
+        char *base = (char *)ctx->ws_pipe[c & 1];
+        void *d_rec = base;
+        double *d_fs = h_fs ? (double *)(base + rec_b) : nullptr;
+        int32_t *d_idx = h_idx ? (int32_t *)(base + rec_b + fs_b) : nullptr;
+        double *d_col[5] = {};
+        char *p = base + rec_b + fs_b + idx_b;
+        for (int i = 0; i < 5; ++i)
+            if (h_col[i]) {
+                d_col[i] = (double *)p;
+                p += col_b;
+            }
+        APDA_CUDA(cudaMemcpyAsync(d_rec, (const char *)h_rec + (size_t)done * rec_bytes, (size_t)cnt * rec_bytes,
+                                  cudaMemcpyHostToDevice, st));
+        if (d_fs) APDA_CUDA(cudaMemcpyAsync(d_fs, h_fs + done, (size_t)cnt * 8, cudaMemcpyHostToDevice, st));
+        APDA_TRY(launch_present_columns(ctx, st, d_rec, rec_cap, cnt, n, fs, d_fs, flexible, k, d_idx, d_col[0], d_col[1],
+                                        d_col[2], d_col[3], d_col[4]));
+        const size_t slots = (size_t)cnt * k, first = (size_t)done * k;
+        if (h_idx) APDA_CUDA(cudaMemcpyAsync(h_idx + first, d_idx, slots * 4, cudaMemcpyDeviceToHost, st));
+        for (int i = 0; i < 5; ++i)
+            if (h_col[i]) APDA_CUDA(cudaMemcpyAsync(h_col[i] + first, d_col[i], slots * 8, cudaMemcpyDeviceToHost, st));
+        return APDA_OK;
+    };
+    int status = APDA_OK;
+    int c = 0;
+    for (int64_t done = 0; done < batch && status == APDA_OK; ++c) {
+        const int64_t cnt = std::min<int64_t>(chunk, batch - done);
+        status = run_chunk(c, done, cnt);
+        done += cnt;
+    }
+    cudaError_t e0 = cudaStreamSynchronize(ctx->pipe[0]);
+    cudaError_t e1 = cudaStreamSynchronize(ctx->pipe[1]);
+    if (status != APDA_OK) return status;
+    if (e0 != cudaSuccess) return apda_cuda_fail(e0, "present_host (stream 0)");
+    if (e1 != cudaSuccess) return apda_cuda_fail(e1, "present_host (stream 1)");
+    return APDA_OK;
+}
+
+extern "C" int apda_fleet_jsonl_dev(apda_ctx *ctx, const void *d_rec, int rec_cap, int64_t batch, int64_t n, double fs,
+                                    const double *d_fs, int flexible, int k, int64_t first_window, char *d_text,
+                                    int64_t text_cap, int64_t *d_offsets) {
+    APDA_TRY(check_present_args(ctx, d_rec, rec_cap, batch, n, k, first_window));
+    if (!d_text || !d_offsets) {
+        apda_set_error("fleet_jsonl: NULL text or offsets");
+        return APDA_ERR_INVALID;
+    }
+    // the exact size is only known on the device: the buffer must hold the bound of every row
+    if (text_cap < 0 || text_cap / APDA_JSONL_ROW_BYTES(k) < batch) {
+        apda_set_error("fleet_jsonl_dev: text_cap %lld < batch (%lld) * APDA_JSONL_ROW_BYTES(%d) = %lld bytes",
+                       (long long)text_cap, (long long)batch, k, (long long)(batch * APDA_JSONL_ROW_BYTES(k)));
+        return APDA_ERR_INVALID;
+    }
+    APDA_CUDA(cudaSetDevice(ctx->device));
+    if (batch == 0) return APDA_OK;
+    auto &l = ctx->stream_lists[ctx->stream];
+    const size_t need = fleet_jsonl_scratch_bytes(batch);
+    if (need > l.jsonl_bytes) {
+        APDA_CUDA(cudaStreamSynchronize(ctx->stream));  // the old scratch may still be in use on this stream
+        APDA_TRY(apda_reserve((void **)&l.jsonl, &l.jsonl_bytes, need));
+    }
+    return launch_fleet_jsonl(ctx, ctx->stream, d_rec, rec_cap, batch, n, fs, d_fs, flexible, k, first_window, d_text,
+                              d_offsets, l.jsonl);
+}
+
+extern "C" int apda_fleet_jsonl_host(apda_ctx *ctx, const void *h_rec, int rec_cap, int64_t batch, int64_t n, double fs,
+                                     const double *h_fs, int flexible, int k, int64_t first_window, char *h_text,
+                                     int64_t text_cap, int64_t *h_offsets) {
+    APDA_TRY(check_present_args(ctx, h_rec, rec_cap, batch, n, k, first_window));
+    if (!h_text || !h_offsets || text_cap < 0) {
+        apda_set_error("fleet_jsonl: NULL text or offsets, or text_cap < 0");
+        return APDA_ERR_INVALID;
+    }
+    APDA_CUDA(cudaSetDevice(ctx->device));
+    h_offsets[0] = 0;
+    if (batch == 0) return APDA_OK;
+    const size_t rec_bytes = (size_t)APDA_REC_BYTES(rec_cap), row_bytes = (size_t)APDA_JSONL_ROW_BYTES(k);
+    const size_t per_window = rec_bytes + (h_fs ? 8 : 0) + 8 + row_bytes;
+    const int64_t chunk = std::min<int64_t>(batch, std::max<int64_t>(1, (int64_t)((96u << 20) / per_window)));
+    const size_t rec_b = align256((size_t)chunk * rec_bytes), fs_b = h_fs ? align256((size_t)chunk * 8) : 0;
+    const size_t off_b = align256((size_t)(chunk + 1) * 8), scan_b = align256(fleet_jsonl_scratch_bytes(chunk));
+    const size_t total = rec_b + fs_b + off_b + scan_b + (size_t)chunk * row_bytes;
+    cudaStream_t st = ctx->pipe[0];
+    if (total > ctx->ws_pipe_bytes[0]) {
+        APDA_CUDA(cudaStreamSynchronize(st));
+        APDA_TRY(apda_reserve(&ctx->ws_pipe[0], &ctx->ws_pipe_bytes[0], total));
+    }
+    char *base = (char *)ctx->ws_pipe[0];
+    void *d_rec = base;
+    double *d_fs = h_fs ? (double *)(base + rec_b) : nullptr;
+    int64_t *d_off = (int64_t *)(base + rec_b + fs_b);
+    int64_t *d_scan = (int64_t *)(base + rec_b + fs_b + off_b);
+    char *d_text = base + rec_b + fs_b + off_b + scan_b;
+    std::vector<int64_t> off((size_t)chunk + 1);
+    // one chunk at a time: its rows' total decides whether (and where) its text may be copied out; every error path
+    // drains the stream before the host buffers go
+    int64_t written = 0;
+    for (int64_t done = 0; done < batch;) {
+        const int64_t cnt = std::min<int64_t>(chunk, batch - done);
+        int status = [&]() -> int {
+            APDA_CUDA(cudaMemcpyAsync(d_rec, (const char *)h_rec + (size_t)done * rec_bytes, (size_t)cnt * rec_bytes,
+                                      cudaMemcpyHostToDevice, st));
+            if (d_fs) APDA_CUDA(cudaMemcpyAsync(d_fs, h_fs + done, (size_t)cnt * 8, cudaMemcpyHostToDevice, st));
+            APDA_TRY(launch_fleet_jsonl(ctx, st, d_rec, rec_cap, cnt, n, fs, d_fs, flexible, k, first_window + done,
+                                        d_text, d_off, d_scan));
+            APDA_CUDA(cudaMemcpyAsync(off.data(), d_off, (size_t)(cnt + 1) * 8, cudaMemcpyDeviceToHost, st));
+            return APDA_OK;
+        }();
+        cudaError_t e = cudaStreamSynchronize(st);
+        if (status != APDA_OK) return status;
+        if (e != cudaSuccess) return apda_cuda_fail(e, "fleet_jsonl_host");
+        if (off[(size_t)cnt] > text_cap - written) {
+            apda_set_error("fleet_jsonl_host: text_cap %lld is smaller than the %lld bytes of rows 0 .. %lld",
+                           (long long)text_cap, (long long)(written + off[(size_t)cnt]), (long long)(done + cnt - 1));
+            return APDA_ERR_INVALID;
+        }
+        status = [&]() -> int {
+            APDA_CUDA(cudaMemcpyAsync(h_text + written, d_text, (size_t)off[(size_t)cnt], cudaMemcpyDeviceToHost, st));
+            return APDA_OK;
+        }();
+        e = cudaStreamSynchronize(st);
+        if (status != APDA_OK) return status;
+        if (e != cudaSuccess) return apda_cuda_fail(e, "fleet_jsonl_host");
+        for (int64_t i = 1; i <= cnt; ++i) h_offsets[done + i] = written + off[(size_t)i];
+        written += off[(size_t)cnt];
+        done += cnt;
+    }
+    return APDA_OK;
 }
 
 // ---------------------------------------------------------------------------------------------------------------

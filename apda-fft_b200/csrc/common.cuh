@@ -47,6 +47,8 @@ struct apda_ctx {
         size_t repair_bytes = 0;
         int *ties = nullptr;  // fp32 tie resolver: windows whose record status is APDA_STATUS_FP32_TIE
         size_t ties_bytes = 0;
+        int64_t *jsonl = nullptr;  // fleet JSONL rows: per-block byte counts, then their prefixes
+        size_t jsonl_bytes = 0;
     };
     std::map<cudaStream_t, StreamLists> stream_lists;
     int generic_only = 0;  // debug/test switch: bypass the specialised fp32 kernels
@@ -175,6 +177,14 @@ size_t resolve_ties_slot_bytes(apda_ctx *ctx, int64_t N, int64_t batch);
 int launch_resolve_ties(apda_ctx *ctx, cudaStream_t st, const float *d_samples, const int *d_nv, int64_t n_samples,
                         int64_t ld, int64_t batch, int64_t N, int center, int flexible, double fs, const double *d_fs,
                         int k, int rec_cap, void *d_rec, int *d_list, void *d_slots);
+// record presentation (present.cu): reference-rounded columns, fleet JSONL rows (d_scratch: fleet_jsonl_scratch_bytes)
+int launch_present_columns(apda_ctx *ctx, cudaStream_t st, const void *d_rec, int rec_cap, int64_t batch, int64_t n,
+                           double fs, const double *d_fs, int flexible, int k, int32_t *d_idx, double *d_freq,
+                           double *d_mag, double *d_prom, double *d_damp, double *d_q);
+size_t fleet_jsonl_scratch_bytes(int64_t batch);
+int launch_fleet_jsonl(apda_ctx *ctx, cudaStream_t st, const void *d_rec, int rec_cap, int64_t batch, int64_t n, double fs,
+                       const double *d_fs, int flexible, int k, int64_t first_window, char *d_text, int64_t *d_offsets,
+                       int64_t *d_scratch);
 
 // ---------------------------------------------------------------------------------------------------------------
 // device side

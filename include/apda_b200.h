@@ -279,6 +279,40 @@ int apda_resolve_fp32_ties_host(apda_ctx *ctx, const float *h_samples, const int
                                 int64_t n_samples, int64_t ld, int64_t batch, int64_t N, int flags, int flexible,
                                 double fs, const double *h_fs, int k, int rec_cap, void *h_rec);
 
+/* ---- record presentation (SURVEY.md 8f rank 4) -----------------------------------------------------------------
+ * What the reference's consumers read, computed from a record table (d_rec: batch records of APDA_REC_BYTES(rec_cap),
+ * 8-byte aligned) with Python's float semantics; fs: one rate for all windows when d_fs / h_fs is NULL; n: the transform
+ * length the records were picked at (a power of two from 4 to 2^30).  Record statuses are not looked at.
+ * apda_present_*: columns of batch x k values, slot j of window w at [w * k + j]; a NULL column is not written.  For
+ * j < min(count, k), with df = fs / n, fn = idx * df, q = fn / (width_bins * df), damping = 1 / (2 * q), each operation
+ * rounded on its own:
+ *   flexible != 0 (utils/get_peak_prominence.py:187-194, records.prominence_dicts): freq = round(fn, 4),
+ *     mag = round(mag, 4), prominence raw, damping = round(damping * 100, 2), q = round(q, 2)
+ *   flexible == 0 (utils/get_peak_resolution.py:113, records.resolution_dicts): freq = fn, mag raw; prominence, damping
+ *     and q are NaN
+ * round() is CPython's (correctly rounded decimal, half to even on the exact binary value).  Where Python would raise
+ * ZeroDivisionError (idx 0 or fs 0 in the flexible picker) the IEEE quotient is written.  Other slots: idx -1, NaN.
+ * apda_fleet_jsonl_*: records.write_fleet_jsonl's text, byte for byte: row w is json.dumps({"window": first_window + w,
+ * "fft_freqs": [...], "fft_mags": [...]}) + "\n" with the freq / mag above, padded with 0.0 to k entries.  Rows are
+ * packed; row w is text[offsets[w] .. offsets[w + 1]), offsets[0] = 0, offsets[batch] = bytes written.
+ *   _dev: text_cap >= batch * APDA_JSONL_ROW_BYTES(k) (the exact size is only known on the device)
+ *   _host: text_cap >= the exact size; otherwise APDA_ERR_INVALID, and no byte past text_cap is written
+ * _dev enqueues on the context stream and does not synchronise the host (except when it grows its scratch, as the other
+ * _dev calls do); a batch of 0 launches nothing. */
+#define APDA_JSONL_ROW_BYTES(k) (64 + 52 * (int64_t)(k))  /* bound on one row: 24 bytes per float, 19 per window number */
+int apda_present_dev(apda_ctx *ctx, const void *d_rec, int rec_cap, int64_t batch, int64_t n, double fs,
+                     const double *d_fs, int flexible, int k, int32_t *d_idx, double *d_freq, double *d_mag,
+                     double *d_prominence, double *d_damping, double *d_q);
+int apda_present_host(apda_ctx *ctx, const void *h_rec, int rec_cap, int64_t batch, int64_t n, double fs,
+                      const double *h_fs, int flexible, int k, int32_t *h_idx, double *h_freq, double *h_mag,
+                      double *h_prominence, double *h_damping, double *h_q);
+int apda_fleet_jsonl_dev(apda_ctx *ctx, const void *d_rec, int rec_cap, int64_t batch, int64_t n, double fs,
+                         const double *d_fs, int flexible, int k, int64_t first_window, char *d_text, int64_t text_cap,
+                         int64_t *d_offsets);
+int apda_fleet_jsonl_host(apda_ctx *ctx, const void *h_rec, int rec_cap, int64_t batch, int64_t n, double fs,
+                          const double *h_fs, int flexible, int k, int64_t first_window, char *h_text, int64_t text_cap,
+                          int64_t *h_offsets);
+
 /* ---- picker helpers on a magnitude array (module-public functions of the reference) --------------------------
  * utils/get_peak_prominence.py:32-54 calculate_prominence(magnitudes, peak_idx) */
 int apda_prominence_f64_host(apda_ctx *ctx, const double *h_mags, int64_t n, int64_t idx, double *out);
